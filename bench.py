@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — audio-frames/sec (fwd+bwd[+all-reduce]+Adam) of SpeechTransformer-base on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (libb200st)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path (libb200st)
   python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm's CPU path (oracle port)
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N   # one rank per GPU, NCCL
 
@@ -208,14 +208,15 @@ def cpu_baseline_object(steps, warmup):
     utterance rather than stalling the bench."""
     threads = cpu_threads()
     T, L = WORKLOAD["T"], WORKLOAD["L"]
-    for (B, Tn, Ln, budget) in ((2, T, L, 150), (1, T // 4, L // 4, 90)):
+    scale = max(1.0, steps / 3.0)              # the budgets below are sized for 3 timed steps
+    for (B, Tn, Ln, budget) in ((2, T, L, 150 * scale), (1, T // 4, L // 4, 90 * scale)):
         r = cpu_sample(B, Tn, Ln, steps, warmup, threads, budget)
         if r is not None:
             sample = "oracle port (fp32 torch-CPU restatement of the reference graph) fwd+bwd, dropout on, B=%d x T=%d frames " \
                      "per step, median of %d step(s) after %d warm-up" % (B, Tn, steps, warmup)
             obj = {"value": B * Tn / r["sec"], "unit": "frames/s", "cores": threads, "kind": "port", "sample": sample}
             # beside it: the unmodified reference itself, for the part of the step it can run (forward only)
-            rf = cpu_sample(B, Tn, Ln, steps, warmup, threads, 90, which="--cpu-ref-worker")
+            rf = cpu_sample(B, Tn, Ln, steps, warmup, threads, 90 * scale, which="--cpu-ref-worker")
             if rf is not None and rf.get("sec"):
                 obj["reference_forward"] = {"value": B * Tn / rf["sec"], "unit": "frames/s (forward only)", "kind": "reference", "cores": threads,
                                             "sample": "unmodified reference neurst_pt.SpeechTransformer.forward(is_training=True) staged under oracle/_ref "
@@ -228,7 +229,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     cpu, sec, shape = cpu_baseline_object(steps, warmup)
     if cpu is None:
         print(json.dumps({"impl": "reference", "unavailable": "CPU oracle sample exceeded its time budget on this host"}), flush=True)
@@ -307,20 +308,23 @@ def encoder_block_roofline(WL, dtype, peaks, iters=20):
 
 
 def run_decode(args):
-    """BASELINE configs[4] (cfg-5): greedy decode of one [1,2000,80] utterance, speech_transformer_s, 200 steps."""
+    """BASELINE configs[4] (cfg-5): greedy decode of one [1,2000,80] utterance, speech_transformer_s, 200 tokens.
+    One step = one whole search (encoder pass + cache build + 200 tokens); --steps searches are timed per precision."""
+    import numpy as np
     import torch
     from neurst_b200 import lib, decode as D
     from neurst_b200.models import SpeechTransformer, speech_transformer_hparams
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product path has no CPU fallback")
     lib.load()
-    V, T, steps = 8192, 2000, 200
+    V, T, n_tok = 8192, 2000, 200
+    steps, warmup = args.steps, max(1, args.warmup)
     sampler = ClockSampler(0)
     sampler.start()
     t_w0 = time.time()
     hp = dict(speech_transformer_hparams("speech_transformer_s")["model.params"])
     tm = {"vocab_size": V, "eos_id": V - 1, "bos_id": V - 2, "unk_id": V - 3}
-    out = {}
+    out, dumped = {}, {}
     for dtype, shadow in (("fp32", False), ("fp16", True)):
         model = SpeechTransformer.new(hp, {"audio_feature_dim": 80, "audio_feature_channels": 1}, tm, precision=dtype)
         model.init_parameters(1234)
@@ -328,55 +332,90 @@ def run_decode(args):
         g = torch.Generator().manual_seed(5)
         src = torch.randn(1, T, 80, 1, generator=g).pin_memory()
         inputs = dict(src=src, src_length=torch.tensor([T]))
-        # never-EOS decoding: minimum_decode_length = steps forces all 200 positions to be decoded
-        kw = dict(maximum_decode_length=steps, extra_decode_length=steps, minimum_decode_length=steps, use_shadow=shadow)
-        for _ in range(2):
+        # never-EOS decoding: minimum_decode_length = n_tok forces all 200 positions to be decoded
+        kw = dict(maximum_decode_length=n_tok, extra_decode_length=n_tok, minimum_decode_length=n_tok, use_shadow=shadow)
+        for _ in range(warmup):
             D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], **kw)
         torch.cuda.synchronize()
-        e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-        e[0].record()
-        enc, bias = D.encode(rt, {k: v.cuda(non_blocking=True) for k, v in inputs.items()})
-        cache = D.create_decoding_cache(rt, enc, bias, steps, shadow)
-        e[1].record()
-        ids, lp, ln = D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], cache=cache, **kw)
-        mode = int(rt.lib.b200st_greedy_used_graph())          # 2 = persistent cooperative kernel
-        host_ids = ids.cpu()
-        e[2].record()
-        torch.cuda.synchronize()
-        enc_ms, dec_ms = e[0].elapsed_time(e[1]), e[1].elapsed_time(e[2])
+        enc_ms = dec_ms = 0.0
+        for _ in range(steps):
+            e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+            e[0].record()
+            enc, bias = D.encode(rt, {k: v.cuda(non_blocking=True) for k, v in inputs.items()})
+            cache = D.create_decoding_cache(rt, enc, bias, n_tok, shadow)
+            e[1].record()
+            ids, lp, ln = D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], cache=cache, **kw)
+            mode = int(rt.lib.b200st_greedy_used_graph())          # 2 = persistent cooperative kernel
+            host_ids = ids.cpu()
+            e[2].record()
+            torch.cuda.synchronize()
+            enc_ms += e[0].elapsed_time(e[1]) / steps
+            dec_ms += e[1].elapsed_time(e[2]) / steps
+        if args.dump_outputs:
+            dumped[dtype + "_token_ids"] = host_ids.numpy().astype(np.float64)
+            dumped[dtype + "_log_probs"] = lp.detach().cpu().numpy().astype(np.float64)
         # the same search as a per-token CUDA graph (round-2 first version), for the comparison
-        cache2 = D.create_decoding_cache(rt, enc, bias, steps, shadow)
+        cache2 = D.create_decoding_cache(rt, enc, bias, n_tok, shadow)
         D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], cache=cache2, persistent=False, **kw)    # warm-up
-        cache2 = D.create_decoding_cache(rt, enc, bias, steps, shadow)
-        g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        g0.record()
-        D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], cache=cache2, persistent=False, **kw)
-        g1.record()
-        torch.cuda.synchronize()
-        out[dtype] = dict(encode_ms=enc_ms, decode_ms=dec_ms, us_per_token=dec_ms * 1e3 / steps, tokens=int(ln[0]),
+        graph_ms = 0.0
+        for _ in range(steps):
+            cache2 = D.create_decoding_cache(rt, enc, bias, n_tok, shadow)
+            g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            g0.record()
+            D.greedy_search(rt, inputs, tm["bos_id"], tm["eos_id"], tm["unk_id"], cache=cache2, persistent=False, **kw)
+            g1.record()
+            torch.cuda.synchronize()
+            graph_ms += g0.elapsed_time(g1) / steps
+        out[dtype] = dict(encode_ms=enc_ms, decode_ms=dec_ms, us_per_token=dec_ms * 1e3 / n_tok, tokens=int(ln[0]),
                           weights="16-bit shadow" if shadow else "fp32 master", mode=mode,
-                          us_per_token_graph_replay=g0.elapsed_time(g1) * 1e3 / steps)
+                          us_per_token_graph_replay=graph_ms * 1e3 / n_tok)
     sampler.mark(t_w0, time.time())
     sampler.stop()
+    if dumped:
+        write_outputs(args.dump_outputs, dumped)
     wbytes = 10.8e6          # decoder + tied embedding parameters read per token
     peaks = load_peaks()
     best = out["fp16"]
     floor_us = wbytes * 2 / (peaks["hbm_gbs"] * 1e9) * 1e6
     line = {"metric": "greedy_decode_tokens_per_sec", "value": 1e6 / best["us_per_token"], "unit": "tokens/s", "n_gpus": 1,
-            "steps": steps, "warmup": 2, "ms_per_step": best["us_per_token"] / 1e3, "higher_is_better": True, "scaling": "weak",
-            "vs_baseline": None, "dtype": "fp32 arithmetic, fp16 weights (fp32-weight variant alongside)", "data": "synthetic",
-            "config": {"workload": "cfg-5: speech_transformer_s greedy decode, one utterance [1,2000,80], 200 steps, preallocated "
-                                   "KV caches, ONE persistent cooperative kernel for the whole search", "per_precision": out},
+            "steps": steps, "warmup": warmup, "ms_per_step": best["encode_ms"] + best["decode_ms"], "higher_is_better": True,
+            "scaling": "weak", "vs_baseline": None, "dtype": "fp32 arithmetic, fp16 weights (fp32-weight variant alongside)",
+            "data": "synthetic",
+            "config": {"workload": "cfg-5: speech_transformer_s greedy decode, one utterance [1,2000,80], 200 tokens, preallocated "
+                                   "KV caches, ONE persistent cooperative kernel for the whole search; one step = one search",
+                       "tokens_per_step": n_tok, "per_precision": out},
             "roofline": {"bound": "hbm", "achieved": wbytes * 2 / (best["us_per_token"] * 1e-6) / 1e9, "peak": peaks["hbm_gbs"],
                          "unit": "GB/s", "frac": floor_us / best["us_per_token"], "traffic": None,
                          "note": "algorithmic bytes per token = 21.6 MB of 16-bit decoder + embedding weights (+ 6 MB fp32 cross "
                                  "K/V); floor %.1f us/token" % floor_us},
-            "e2e": {"value": steps / ((best["encode_ms"] + best["decode_ms"]) * 1e-3), "unit": "tokens/s (encoder pass + cache "
-                    "build + 200 steps + ids D2H)", "h2d_bytes_per_step": T * 80 * 4, "d2h_bytes_per_step": steps * 8},
+            "e2e": {"value": n_tok / ((best["encode_ms"] + best["decode_ms"]) * 1e-3), "unit": "tokens/s (encoder pass + cache "
+                    "build + 200 tokens + ids D2H)", "h2d_bytes_per_step": T * 80 * 4, "d2h_bytes_per_step": n_tok * 8},
             "clocks": sampler.summary(),
             "gpu_launches": 2}
     print(json.dumps(line), flush=True)
 
+
+# --dump-outputs: a fixed sample of the fp32 master parameters (16 MB) keeps the dump well under 64 MB at every workload
+DUMP_PARAM_SAMPLES = 4 << 20
+
+
+def timed_step_outputs(trainer, loss):
+    """Host copies of what a training step leaves its caller: the loss it returns and the parameters its Adam update
+    wrote (a seeded sample of the flat fp32 arena, in arena order, so two builds can be compared element for element)."""
+    import numpy as np
+    import torch
+    params = trainer.rt.params.detach().reshape(-1)
+    n = params.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_PARAM_SAMPLES), replace=False))
+    sample = params[torch.from_numpy(idx).to(params.device)].float().cpu().numpy()
+    return {"loss": np.array([float(loss)], dtype=np.float64), "params_sample": sample.astype(np.float32)}
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_gpu(args):
@@ -467,6 +506,8 @@ def run_gpu(args):
     sampler.mark(t_w0, time.time())
     launches = lib.launch_count() - launches0
     loss_val = float(losses[-1])
+    # what the last timed step returned, taken before the e2e steps below train the parameters further
+    dumped = timed_step_outputs(trainer, losses[-1]) if args.dump_outputs and rank == 0 else None
     for i in range(2):
         e2e_step(i)
     t_w0 = time.time()
@@ -589,6 +630,8 @@ def run_gpu(args):
         line["roofline"]["encoder_block"] = enc_block
     if cpu:
         line["cpu_baseline"] = cpu
+    if dumped:
+        write_outputs(args.dump_outputs, dumped)
     print(json.dumps(line), flush=True)
     leave(0)
 
@@ -608,7 +651,14 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS) + ["decode"],
                     help="cfg2 = BASELINE headline [32,1000,80]; cfg3 / cfg3w = [8|64,1500,80]; cfg4 = speech_transformer_m ragged buckets; "
                          "decode = cfg-5 greedy decode")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (training: loss and a seeded sample of the "
+                         "updated parameters; decode: token ids and log-probabilities per precision)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is supported by --impl b200")
     if args.cpu_ref_worker:
         cpu_ref_worker(args.cpu_ref_worker)
         return
@@ -627,6 +677,8 @@ def main():
         cmd += ["--dtype", args.dtype, "--workload", args.workload]
         if args.no_cpu_baseline:
             cmd.append("--no-cpu-baseline")
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
         sys.exit(subprocess.call(cmd))
     if args.workload == "decode":
         run_decode(args)

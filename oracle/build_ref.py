@@ -62,9 +62,14 @@ def build(force=False):
     return DEST
 
 
+def reference_root():
+    """The reference tree the oracle loads: the source checkout when present, else the copy staged here (None if neither)."""
+    return SRC if os.path.isdir(os.path.join(SRC, "neurst_pt")) else staged()
+
+
 def reference_speech_transformer(hparams, vocab, seed=1234):
     """Instantiates the unmodified reference `neurst_pt` SpeechTransformer (random init) from the staged tree."""
-    root = staged() or (SRC if os.path.isdir(os.path.join(SRC, "neurst_pt")) else None)
+    root = staged() or reference_root()
     if root is None:
         raise RuntimeError("no reference tree: run oracle/build_ref.py in the build container")
     os.environ["NEURST_REFERENCE"] = root

@@ -1,12 +1,14 @@
-"""ORACLE (test infrastructure only): generates tests/golden/*.npz.  Run in the build container only
-(`python oracle/make_golden.py`); it reads /root/reference, which does not exist on the GPU box.
+"""ORACLE (test infrastructure only): generates the reference-derived fixtures under tests/golden/
+(`NEURST_REFERENCE=<reference checkout> python oracle/make_golden.py`).  The tests read only what it wrote, never the
+reference itself.
 
-Two kinds of fixtures:
+Three kinds of fixtures:
   kat_*.npz   — the TF-generated known-answer vectors hard-coded in the reference's own tests
                 (tests/neurst/**), extracted here by parsing those test files' literals with `ast`
                 (weights, inputs, expected outputs; nothing is executed).
-  refpt_*.npz — inputs, weights (converted to the TF layouts of SURVEY Appx B) and outputs of the
-                UNMODIFIED reference PyTorch mirror (neurst_pt) run on CPU through oracle/ref_shim.py.
+  refpt_*.npz — inputs, weight seed and outputs of the UNMODIFIED reference PyTorch mirror (neurst_pt) run on CPU
+                through oracle/ref_shim.py.
+  ref_bucket_boundaries.json — the reference's length-bucket table at a few arguments.
 """
 import ast
 import os
@@ -131,73 +133,18 @@ def make_kats():
 # ----------------------------------------------------------------------------------------------
 # reference-PT generated fixtures
 # ----------------------------------------------------------------------------------------------
-def pt_speech_transformer_params(model):
-    """Reference PT module -> flat dict in TF layouts (inverse of the map in
-    tests/neurst_pt/models/speech_transformer_test.py:57-152 / SURVEY Appx B)."""
-    import torch
-    P = {}
-
-    def g(t):
-        return t.detach().clone().double().numpy()
-
-    sm = model._src_modality._embedding_layer if hasattr(model._src_modality, "_embedding_layer") else model._src_modality
-    if hasattr(sm, "_conv_layer1"):
-        P["src.conv1.kernel"] = g(sm._conv_layer1.weight.permute(2, 3, 1, 0)); P["src.conv1.bias"] = g(sm._conv_layer1.bias)
-        P["src.conv2.kernel"] = g(sm._conv_layer2.weight.permute(2, 3, 1, 0)); P["src.conv2.bias"] = g(sm._conv_layer2.bias)
-        P["src.ln1.gamma"] = g(sm._norm_layer1.weight); P["src.ln1.beta"] = g(sm._norm_layer1.bias)
-        P["src.ln2.gamma"] = g(sm._norm_layer2.weight); P["src.ln2.beta"] = g(sm._norm_layer2.bias)
-        P["src.dense.kernel"] = g(sm._dense_layer.weight.t()); P["src.dense.bias"] = g(sm._dense_layer.bias)
-
-    def att(pre, wrap, cross):
-        P[pre + ".ln.gamma"] = g(wrap._norm_layer.weight); P[pre + ".ln.beta"] = g(wrap._norm_layer.bias)
-        a = wrap._layer
-        if cross:
-            P[pre + ".q.kernel"] = g(a._q_transform_layer._kernel); P[pre + ".q.bias"] = g(a._q_transform_layer._bias)
-            P[pre + ".kv.kernel"] = g(a._kv_transform_layer._kernel); P[pre + ".kv.bias"] = g(a._kv_transform_layer._bias)
-        else:
-            P[pre + ".qkv.kernel"] = g(a._qkv_transform_layer._kernel); P[pre + ".qkv.bias"] = g(a._qkv_transform_layer._bias)
-        P[pre + ".out.kernel"] = g(a._output_transform_layer._kernel); P[pre + ".out.bias"] = g(a._output_transform_layer._bias)
-
-    def ffn(pre, wrap):
-        P[pre + ".ln.gamma"] = g(wrap._norm_layer.weight); P[pre + ".ln.beta"] = g(wrap._norm_layer.bias)
-        f = wrap._layer
-        P[pre + ".w1"] = g(f._dense1.weight.t()); P[pre + ".b1"] = g(f._dense1.bias)
-        P[pre + ".w2"] = g(f._dense2.weight.t()); P[pre + ".b2"] = g(f._dense2.bias)
-
-    for i, layer in enumerate(model._encoder._stacking_layers):
-        att("enc.%d.att" % i, layer[0], False); ffn("enc.%d.ffn" % i, layer[1])
-    P["enc.out_ln.gamma"] = g(model._encoder._output_norm_layer.weight)
-    P["enc.out_ln.beta"] = g(model._encoder._output_norm_layer.bias)
-    for i, layer in enumerate(model._decoder._stacking_layers):
-        att("dec.%d.self" % i, layer[0], False); att("dec.%d.cross" % i, layer[1], True); ffn("dec.%d.ffn" % i, layer[2])
-    P["dec.out_ln.gamma"] = g(model._decoder._output_norm_layer.weight)
-    P["dec.out_ln.beta"] = g(model._decoder._output_norm_layer.bias)
-    tm = model._trg_modality._embedding_layer
-    P["trg.emb"] = g(tm._shared_weights); P["trg.bias"] = g(tm._bias)
-    return P
-
-
-def _all_reference_params(model):
-    """The reference keeps layer stacks in python lists (invisible to .parameters()); walk them explicitly."""
-    import torch
-    ps = list(model.parameters())
-    for stack in (model._encoder._stacking_layers, model._decoder._stacking_layers):
-        for layer in stack:
-            for sub in layer:
-                if sub is not None:
-                    ps.extend(sub.parameters())
-    return ps
-
-
 def make_refpt():
+    """Weights are `restatement.init_params(cfg, seed, random_bias=True)`, copied into the reference module through
+    neurst_b200.checkpoints.to_reference_pt; the fixture stores the seed instead of the weights (tests/golden_utils.py
+    regenerates them), which keeps it small and pins the weight map along with the forward."""
     import torch
     from oracle import ref_shim
+    from oracle import restatement as R
+    from neurst_b200 import checkpoints as CK
     ref_shim.install()
     from neurst_pt.models.speech_transformer import SpeechTransformer
 
     def build(d, heads, enc_layers, dec_layers, ffn_size, channels, vocab, seed):
-        torch.manual_seed(seed)
-        np.random.seed(seed)
         params = {
             "modality.source.kernel_size": 3, "modality.source.strides": 2, "modality.source.channels": channels,
             "modality.source.layer_norm": True, "modality.dim": d, "modality.source.dim": None,
@@ -212,13 +159,14 @@ def make_refpt():
                            side + ".layer_postprocess_epsilon": 1e-6})
         src_meta = {"audio_feature_dim": 80, "audio_feature_channels": 1}
         trg_meta = {"vocab_size": vocab, "eos_id": vocab - 1, "bos_id": vocab - 2, "unk_id": vocab - 3}
+        cfg = dict(model="speech", d=d, heads=heads, enc_layers=enc_layers, dec_layers=dec_layers, ffn=ffn_size,
+                   channels=channels, feat=80, in_channels=1, vocab=vocab)
+        P = R.init_params(cfg, seed=seed, random_bias=True)
         with torch.no_grad():
             model = SpeechTransformer.new(params, src_meta, trg_meta)
-            # make every bias / LN parameter non-trivial so the fixtures exercise them
-            g = torch.Generator().manual_seed(seed + 1)
-            for p in _all_reference_params(model):
-                if p.dim() == 1:
-                    p.add_(0.1 * torch.randn(p.shape, generator=g))
+            CK.to_reference_pt(P, model)
+        back = CK.from_reference_pt(model)
+        assert set(back) == set(P) and all(torch.equal(back[k], P[k]) for k in P)
         return model
 
     cases = [
@@ -241,16 +189,35 @@ def make_refpt():
             sm = model._src_modality
             emb = sm(src.clone())
             conv = sm._embedding_layer(src.clone())
-        P = pt_speech_transformer_params(model)
         np.savez(os.path.join(OUT, name + ".npz"), src=src.numpy(), src_length=lengths.numpy(),
                  trg_input=trg_input.numpy(), logits=logits.numpy(), emb=emb.numpy(), conv=conv.numpy(),
                  cfg=np.array([mk["d"], mk["heads"], mk["enc_layers"], mk["dec_layers"], mk["ffn_size"], mk["channels"],
-                               mk["vocab"]]),
-                 **{"P:" + k: v.astype(np.float32) for k, v in P.items()})
+                               mk["vocab"]]), seed=np.array(mk["seed"]))
         print(name, "logits", tuple(logits.shape))
+
+
+# ----------------------------------------------------------------------------------------------
+# reference functions evaluated at fixed arguments
+# ----------------------------------------------------------------------------------------------
+BUCKET_ARGS = [(3000, 128), (2000, 100), (800, None), (3000, 300)]
+
+
+def make_bucket_boundaries():
+    """neurst/tasks/speech2text.py `create_audio_bucket_boundaries`, loaded from the source with `ast` (the module itself
+    imports TensorFlow) and evaluated at BUCKET_ARGS."""
+    import json
+    import math
+    src = open(os.path.join(REF, "neurst/tasks/speech2text.py")).read()
+    fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "create_audio_bucket_boundaries")
+    ns = {"math": math}
+    exec(compile(ast.Module([fn], []), "ref", "exec"), ns)
+    cases = [{"maxlen": a, "minlen": b, "boundaries": ns["create_audio_bucket_boundaries"](a, b)} for a, b in BUCKET_ARGS]
+    with open(os.path.join(OUT, "ref_bucket_boundaries.json"), "w") as f:
+        json.dump({"source": "reference neurst/tasks/speech2text.py create_audio_bucket_boundaries", "cases": cases}, f, indent=1)
 
 
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     make_kats()
     make_refpt()
+    make_bucket_boundaries()

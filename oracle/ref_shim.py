@@ -1,10 +1,11 @@
-"""ORACLE (test infrastructure only): import shim that loads the UNMODIFIED reference PyTorch mirror
-`/root/reference/neurst_pt` in the build container (TensorFlow is not installed; SURVEY.md §8c).
+"""ORACLE (test infrastructure only): import shim that loads the UNMODIFIED reference PyTorch mirror `neurst_pt`
+from $NEURST_REFERENCE, the reference checkout or the copy of it oracle/build_ref.py stages under oracle/_ref
+(TensorFlow is not installed; SURVEY.md §8c).
 
 It installs a fake `tensorflow` module exposing the few symbols neurst_pt / neurst.utils touch
 (tf.nest, tf.io.gfile, tf.errors.OpError), pre-seeds `neurst` / `neurst.utils` as namespace packages so that
 neurst/__init__.py (which imports every TF sub-package) is never executed, and stubs `neurst.utils.compat`.
-/root/reference does not exist on the GPU box: only oracle/make_golden.py (run here) uses this shim.
+Users: oracle/make_golden.py, the registry plug-in and weight-map tests, bench.py's reference CPU leg.
 """
 import importlib
 import os
@@ -12,7 +13,9 @@ import shutil
 import sys
 import types
 
-REF = os.environ.get("NEURST_REFERENCE", "/root/reference")
+from oracle import build_ref
+
+REF = os.environ.get("NEURST_REFERENCE") or build_ref.reference_root() or ""
 
 
 def _flatten(x):
@@ -52,7 +55,7 @@ def _map_structure(fn, *structs, **kwargs):
 
 def install():
     if not os.path.isdir(REF):
-        raise RuntimeError("reference tree not found at %s (the shim only works in the build container)" % REF)
+        raise RuntimeError("no reference tree: neither NEURST_REFERENCE nor a copy staged by oracle/build_ref.py")
     if "tensorflow" not in sys.modules:
         tf = types.ModuleType("tensorflow")
         nest = types.ModuleType("tensorflow.nest")

@@ -8,6 +8,8 @@ Stored: per file the record count and a SHA-256 over the record payloads; the fi
 (hex, 16 framing bytes + payload each) with the ids an INDEPENDENT decoder (the google.protobuf runtime on a descriptor
 built from the published example.proto / feature.proto) reads from them, and the text those ids spell in the reference's
 vocabulary (vocab.en) — which is line 4 / line 5 of train.example.en.tok.bpe.txt, the text the records were made from.
+Beside the JSON, a sample of the fixture itself: shard 0 and vocab.en gzipped, and a 64-bit digest of every line of
+train.example.en.tok.bpe.txt (line_digest) in place of the text.
 """
 import glob
 import hashlib
@@ -55,6 +57,22 @@ def example_class():
     return message_factory.GetMessageClass(pool.FindMessageTypeByName("b200st_tf.Example"))
 
 
+def line_digest(text):
+    """First 8 bytes of the SHA-256 of a UTF-8 line, as an unsigned little-endian integer."""
+    return int.from_bytes(hashlib.sha256(text.encode("utf-8")).digest()[:8], "little")
+
+
+def write_samples(lines):
+    import gzip
+    import numpy as np
+    gold = os.path.join(ROOT, "tests", "golden")
+    shard0 = sorted(glob.glob(os.path.join(EX, "train.tfrecords-*")))[0]
+    for src, dst in ((shard0, "ref_" + os.path.basename(shard0) + ".gz"), (os.path.join(EX, "vocab.en"), "ref_vocab.en.gz")):
+        with open(src, "rb") as fi, gzip.GzipFile(os.path.join(gold, dst), "wb", mtime=0) as fo:
+            fo.write(fi.read())
+    np.save(os.path.join(gold, "ref_train_en_line_digests.npy"), np.array(sorted(line_digest(l) for l in lines), np.uint64))
+
+
 def main():
     import numpy as np
     from neurst_b200 import tfrecord as R
@@ -83,6 +101,7 @@ def main():
         pos += 16 + ln
     with open(os.path.join(ROOT, "tests", "golden", "tfrecord_fixture.json"), "w") as fo:
         json.dump(out, fo, indent=1)
+    write_samples(lines)
     print(json.dumps(out["files"], indent=1))
     print([(r["label_text_line"], r["label_text"]) for r in out["records"]])
 

@@ -61,9 +61,12 @@ def kat_params(kat, cfg, default_stack, dtype=torch.float32):
 
 
 def refpt_case(name, dtype=torch.float32):
+    """Fixture, weights and config of a refpt_* case.  The fixture stores the weight seed: the reference ran on
+    oracle.restatement.init_params(cfg, seed, random_bias=True), regenerated here bit for bit."""
+    from oracle import restatement as R
     z = load(name)
-    P = {k[2:]: t(v, dtype) for k, v in z.items() if k.startswith("P:")}
     d, heads, enc_layers, dec_layers, ffn, channels, vocab = [int(x) for x in z["cfg"]]
     cfg = dict(model="speech", d=d, heads=heads, enc_layers=enc_layers, dec_layers=dec_layers, ffn=ffn,
                channels=channels, feat=80, in_channels=1, vocab=vocab)
+    P = {k: v.to(dtype) for k, v in R.init_params(cfg, seed=int(z["seed"]), random_bias=True).items()}
     return z, P, cfg

@@ -1,5 +1,5 @@
 """CPU tests of the f3 / f4 rows: reference variable names, npz round trip, neurst_pt weight map (against the unmodified
-reference module when /root/reference exists), bucket table vs the reference function, SpecAugment sampling rule."""
+reference module, from the copy oracle/build_ref.py stages), bucket table vs the reference function, SpecAugment sampling rule."""
 import os
 
 import numpy as np
@@ -8,10 +8,12 @@ import torch
 
 from neurst_b200 import checkpoints as CK
 from neurst_b200 import data as D
+from oracle import build_ref
 from oracle import restatement as R
 
-REF = os.environ.get("NEURST_REFERENCE", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+# the reference checkout, or the unmodified copy of it that build() stages under oracle/_ref
+REF = os.environ.get("NEURST_REFERENCE") or build_ref.reference_root()
+needs_ref = pytest.mark.skipif(not REF, reason="no reference tree and no copy staged by oracle/build_ref.py")
 
 
 class _FakeRT:
@@ -94,15 +96,13 @@ def test_weight_map_against_the_unmodified_reference_module():
     assert float((ref - mine).abs().max()) < 1e-4
 
 
-@needs_ref
 def test_bucket_boundaries_match_the_reference_function():
-    import ast
-    src = open(os.path.join(REF, "neurst/tasks/speech2text.py")).read()
-    fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "create_audio_bucket_boundaries")
-    ns = {"math": __import__("math")}
-    exec(compile(ast.Module([fn], []), "ref", "exec"), ns)
-    for maxlen, minlen in ((3000, 128), (2000, 100), (800, None), (3000, 300)):
-        assert D.create_audio_bucket_boundaries(maxlen, minlen) == ns["create_audio_bucket_boundaries"](maxlen, minlen)
+    # the reference function's own outputs (tests/golden/ref_bucket_boundaries.json, oracle/make_golden.py)
+    import json
+    cases = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_bucket_boundaries.json")))["cases"]
+    assert len(cases) == 4
+    for c in cases:
+        assert D.create_audio_bucket_boundaries(c["maxlen"], c["minlen"]) == c["boundaries"]
 
 
 def test_frame_budget_bucketer_shapes_and_batches():
@@ -152,8 +152,8 @@ def test_staged_reference_copy_is_unmodified_and_runs():
     assert len(man) > 20 and "neurst_pt/models/speech_transformer.py" in man
     for rel, digest in man.items():
         assert hashlib.sha256(open(os.path.join(root, rel), "rb").read()).hexdigest() == digest
-        if os.path.isdir(REF):
-            assert hashlib.sha256(open(os.path.join(REF, rel), "rb").read()).hexdigest() == digest, rel
+        if os.path.isdir(os.path.join(build_ref.SRC, "neurst_pt")):
+            assert hashlib.sha256(open(os.path.join(build_ref.SRC, rel), "rb").read()).hexdigest() == digest, rel
     code = r'''
 import os, sys, torch
 sys.path.insert(0, %r)

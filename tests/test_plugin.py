@@ -1,13 +1,16 @@
-"""The registry drop-in: with the reference on sys.path (build container only — skipped on the GPU box, where
-/root/reference does not exist) `neurst_b200.plugin.register()` makes the reference's OWN `build_model` return the
+"""The registry drop-in: with the reference on sys.path (the unmodified copy oracle/build_ref.py stages under oracle/_ref)
+`neurst_b200.plugin.register()` makes the reference's OWN `build_model` return the
 libb200st-backed class, through the `class_or_method_args` branch of registry.build_x (neurst/utils/registry.py:90-102)."""
 import os
 
 import pytest
 import torch
 
-REF = os.environ.get("NEURST_REFERENCE", "/root/reference")
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
+from oracle import build_ref
+
+# the reference checkout, or the unmodified copy of it that build() stages under oracle/_ref
+REF = os.environ.get("NEURST_REFERENCE") or build_ref.reference_root()
+needs_ref = pytest.mark.skipif(not REF, reason="no reference tree and no copy staged by oracle/build_ref.py")
 
 
 def _register():

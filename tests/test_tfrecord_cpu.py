@@ -3,9 +3,9 @@ reference's deterministic file interleave / sharding, AudioTFRecordDataset and t
 
 Pins: CRC-32C known answers (RFC 3720 B.4); two records written by TensorFlow, taken verbatim from the reference's own
 fixture (tests/golden/tfrecord_fixture.json, made by tests/golden/make_tfrecord_fixture.py), whose ids were read by an
-independent decoder (google.protobuf runtime) and spell lines of the text the reference built the records from; the whole
-reference fixture when /root/reference is present; the protobuf runtime as a second encoder/decoder of the same schema."""
-import glob
+independent decoder (google.protobuf runtime) and spell lines of the text the reference built the records from; the first
+shard of that fixture, read whole; the protobuf runtime as a second encoder/decoder of the same schema."""
+import gzip
 import hashlib
 import importlib.util
 import json
@@ -20,14 +20,17 @@ from neurst_b200 import tfrecord as R
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = json.load(open(os.path.join(HERE, "golden", "tfrecord_fixture.json")))
-REF_EX = "/root/reference/tests/examples"
 
 
-def _example_class():
+def _fixture_module():
     spec = importlib.util.spec_from_file_location("make_tfrecord_fixture", os.path.join(HERE, "golden", "make_tfrecord_fixture.py"))
     m = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(m)
-    return m.example_class()
+    return m
+
+
+def _example_class():
+    return _fixture_module().example_class()
 
 
 def test_crc32c_known_answers():
@@ -71,26 +74,30 @@ def test_records_written_by_tensorflow(tmp_path):
     assert list(R.read_records(str(p))) == []
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EX), reason="reference tree not present")
-def test_whole_reference_fixture():
-    files = sorted(glob.glob(os.path.join(REF_EX, "train.tfrecords-*")))
-    assert [os.path.basename(f) for f in files] == [g["name"] for g in GOLD["files"]]
-    for f, g in zip(files, GOLD["files"]):
-        h, n = hashlib.sha256(), 0
-        for rec in R.read_records(f, verify=2):
-            h.update(rec.tobytes()); n += 1
-        assert (n, h.hexdigest()) == (g["records"], g["payload_sha256"])
-    # every target of the data the records were built from appears exactly once, EOS-terminated: 7594 lines <-> 7594 records
-    vocab = [l.rstrip("\n").split(" ")[0] for l in open(os.path.join(REF_EX, "vocab.en"), encoding="utf-8")]
-    lines = sorted(l.rstrip("\n") for l in open(os.path.join(REF_EX, "train.example.en.tok.bpe.txt"), encoding="utf-8"))
+def test_reference_fixture_first_shard(tmp_path):
+    """Shard 0 of the reference's TensorFlow-written fixture (stored gzipped under tests/golden) read end to end."""
+    g = GOLD["files"][0]
+    with gzip.open(os.path.join(HERE, "golden", "ref_" + g["name"] + ".gz"), "rb") as f:
+        (tmp_path / g["name"]).write_bytes(f.read())
+    h, n = hashlib.sha256(), 0
+    for rec in R.read_records(str(tmp_path / g["name"]), verify=2):
+        h.update(rec.tobytes()); n += 1
+    assert (n, h.hexdigest()) == (g["records"], g["payload_sha256"])
+    # every target decodes, EOS-terminated, to a line of the text the records were built from (stored as line digests:
+    # 7594 lines <-> 7594 records over the four shards)
+    with gzip.open(os.path.join(HERE, "golden", "ref_vocab.en.gz"), "rt", encoding="utf-8") as f:
+        vocab = [l.rstrip("\n").split(" ")[0] for l in f]
+    lines = np.load(os.path.join(HERE, "golden", "ref_train_en_line_digests.npy"))
+    assert len(lines) == sum(f["records"] for f in GOLD["files"]) == 7594
+    line_digest, lines = _fixture_module().line_digest, set(lines.tolist())
     got = []
-    for el in R.load_tfrecords(os.path.join(REF_EX, "train.tfrecords"), {"feature": R.VarLenInt64, "label": R.VarLenInt64}):
+    for el in R.load_tfrecords(str(tmp_path / "train.tfrecords"), {"feature": R.VarLenInt64, "label": R.VarLenInt64}):
         ids = el["label"]
         assert ids[-1] == len(vocab) + 2                            # EOS id of the reference's vocabulary wrapper
         got.append(" ".join(vocab[i] if i < len(vocab) else "<unk>" for i in ids[:-1]))
-    assert len(got) == len(lines) == 7594
-    same = sum(a == b for a, b in zip(sorted(got), lines))
-    assert same > 0.97 * len(lines)                                 # the rest contain out-of-vocabulary pieces (<unk>)
+    assert len(got) == n
+    same = sum(line_digest(t) in lines for t in got)
+    assert same > 0.97 * n                                          # the rest contain out-of-vocabulary pieces (<unk>)
 
 
 def test_example_codec_against_the_protobuf_runtime():
