@@ -260,10 +260,6 @@ int b200st_gemm_bench(const b200st_gemm_args* args, int32_t iters, float* ms_per
 int b200st_profile_begin(void);
 int b200st_profile_end(double* gemm_ms, double* gemm_flops, int64_t* gemm_launches);
 
-/* tests only: override tcgen05 shared-memory descriptor fields / tile config (0 = default) */
-int b200st_debug_tc(uint32_t mn_lbo, uint32_t mn_sbo, uint32_t k_lbo, uint32_t k_sbo, int32_t force_bn,
-                    int32_t force_stages, int32_t max_ctas);
-
 #ifdef __cplusplus
 }
 #endif

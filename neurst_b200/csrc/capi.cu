@@ -87,14 +87,6 @@ int b200st_profile_end(double* gemm_ms, double* gemm_flops, int64_t* gemm_launch
   return tc_profile_end(gemm_ms, gemm_flops, gemm_launches);
 }
 
-int b200st_debug_tc(uint32_t mn_lbo, uint32_t mn_sbo, uint32_t k_lbo, uint32_t k_sbo, int32_t force_bn,
-                    int32_t force_stages, int32_t max_ctas) {
-  TcDebug& d = tc_debug();
-  d.mn_lbo_bytes = mn_lbo; d.mn_sbo_bytes = mn_sbo; d.k_lbo_bytes = k_lbo; d.k_sbo_bytes = k_sbo;
-  d.force_bn = force_bn; d.force_stages = force_stages; d.max_ctas = max_ctas;
-  return 0;
-}
-
 
 struct b200st_model { Model m; };
 

@@ -246,7 +246,8 @@ __global__ void __launch_bounds__(256, (CPL <= 8 ? 3 : 1)) conv1_fwd_kernel(cons
 // ahead and broadcast with shuffles, each warp walks a contiguous range of positions.
 // SAVE: store xhat + 1/sigma (normalised-save mode); else y = relu(LN(z) * gamma + beta).
 // ---------------------------------------------------------------------------------------------
-// d{0,1} += a * b{0,1} as one packed fp32x2 instruction (FFMA2, sm_100): half the issue slots of two FFMAs
+// d{0,1} += a * b{0,1} as one packed fp32x2 instruction (FFMA2, sm_100): half the issue slots of two FFMAs, and the same
+// rounding (one fma.rn per element); B200 cfg-2 step 6.155 ms vs 6.173 ms with scalar fmaf (profiles/r02_bench_cfg2_ffma2.json)
 __device__ __forceinline__ void ffma2_bcast(float& d0, float& d1, float a, float b0, float b1) {
   uint64_t av, bv, cv;
   asm("mov.b64 %0, {%1, %1};" : "=l"(av) : "f"(a));
@@ -256,7 +257,7 @@ __device__ __forceinline__ void ffma2_bcast(float& d0, float& d1, float a, float
   asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(cv));
 }
 
-template <typename T, bool SAVE, bool F2 = false>
+template <typename T, bool SAVE>
 __global__ void __launch_bounds__(256, 2) conv1_fwd_c256_kernel(const float* __restrict__ src, const float* __restrict__ w,
                                                                 const float* __restrict__ bias, const float* __restrict__ gamma,
                                                                 const float* __restrict__ beta, float eps, T* __restrict__ y,
@@ -312,13 +313,8 @@ __global__ void __launch_bounds__(256, 2) conv1_fwd_c256_kernel(const float* __r
 #pragma unroll
     for (int tp = 0; tp < 9; ++tp) {
       const float x = __shfl_sync(0xffffffffu, xv, tp);
-      if constexpr (F2) {
 #pragma unroll
-        for (int i = 0; i < 8; i += 2) ffma2_bcast(z[i], z[i + 1], x, wreg[tp][i], wreg[tp][i + 1]);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) z[i] = fmaf(x, wreg[tp][i], z[i]);
-      }
+      for (int i = 0; i < 8; i += 2) ffma2_bcast(z[i], z[i + 1], x, wreg[tp][i], wreg[tp][i + 1]);
     }
     float s1 = 0.f;
 #pragma unroll
@@ -767,9 +763,7 @@ static int conv1_fwd_launch(const float* src, const float* w, const float* b, co
   if (vec && C == 256 && Cin == 1 && (use_ln || rstd_out) && ((reinterpret_cast<uintptr_t>(w) & 15) == 0) &&
       ((reinterpret_cast<uintptr_t>(b) & 15) == 0) && (rstd_out || (((reinterpret_cast<uintptr_t>(gamma) | reinterpret_cast<uintptr_t>(beta)) & 15) == 0))) {
     const int grid1 = pick_grid(npos, 8 * 16, 148 * 2);
-    static const bool f2 = getenv("B200ST_NO_CONV1_FFMA2") == nullptr;   // packed fp32x2 FMAs (same rounding: fma.rn per element; 6.155 vs 6.173 ms step)
-    if (rstd_out && f2) DISPATCH_DTYPE(y_dtype, TT, (launch_pdl(conv1_fwd_c256_kernel<TT, true, true>, grid1, 256, 0, s, src, w, b, gamma, beta, eps, (TT*)y1, rstd_out, B, T, F, T1, F1)));
-    else if (rstd_out) DISPATCH_DTYPE(y_dtype, TT, (launch_pdl(conv1_fwd_c256_kernel<TT, true>, grid1, 256, 0, s, src, w, b, gamma, beta, eps, (TT*)y1, rstd_out, B, T, F, T1, F1)));
+    if (rstd_out) DISPATCH_DTYPE(y_dtype, TT, (launch_pdl(conv1_fwd_c256_kernel<TT, true>, grid1, 256, 0, s, src, w, b, gamma, beta, eps, (TT*)y1, rstd_out, B, T, F, T1, F1)));
     else DISPATCH_DTYPE(y_dtype, TT, (launch_pdl(conv1_fwd_c256_kernel<TT, false>, grid1, 256, 0, s, src, w, b, gamma, beta, eps, (TT*)y1, rstd_out, B, T, F, T1, F1)));
     ++g_kernel_launches;
     B200ST_LAUNCH_CHECK();

@@ -85,16 +85,9 @@ int fused_mlp_fwd(const void* X, int dtype, int M, int d, int ffn, const void* W
 int fused_mlp_bwd(const void* dY, int dtype, int M, int d, int ffn, const void* W1, const void* W2, const void* F1, float scale,
                   void* dF1, float* dH, cudaStream_t stream, int* tickets = nullptr);
 
-// Debug knobs for the descriptor probe (tests only). 0 restores defaults.
-struct TcDebug {
-  uint32_t mn_lbo_bytes, mn_sbo_bytes, k_lbo_bytes, k_sbo_bytes;
-  int force_bn;     // 0 = auto
-  int force_stages; // 0 = auto
-  int max_ctas;     // 0 = #SMs
-  int one_cta_per_sm; // 1 = disable the 2-CTAs-per-SM mode of the BN <= 128 variants
-  int reserve_sms;    // SMs left to concurrent communication kernels (set by the model while gradient all-reduces overlap)
-};
-TcDebug& tc_debug();
+// SMs the persistent tcgen05 grids leave to concurrent communication kernels (set by the model while gradient all-reduces
+// overlap the backward pass; 0 = none)
+void gemm_set_reserved_sms(int n);
 int64_t tc_launch_count();
 void tc_count_launch();
 void tc_profile_begin();

@@ -148,19 +148,11 @@ static SideStream& side_stream() {
   static bool init = false;
   if (!init) {
     init = true;
-    if (!getenv("B200ST_NO_SIDE_STREAM")) {
-      // weight gradients are filler work: with B200ST_SIDE_PRIORITY the side stream gets the lowest priority, so CTAs of the
-      // backward chain win whenever both have blocks waiting for an SM
-      int lo = 0, hi = 0;
-      cudaDeviceGetStreamPriorityRange(&lo, &hi);
-      const bool low = getenv("B200ST_SIDE_PRIORITY") != nullptr;
-      ss.ok = (low ? cudaStreamCreateWithPriority(&ss.stream, cudaStreamNonBlocking, lo)
-                   : cudaStreamCreateWithFlags(&ss.stream, cudaStreamNonBlocking)) == cudaSuccess &&
-              cudaEventCreateWithFlags(&ss.fork, cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&ss.done[0], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&ss.done[1], cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&ss.bits_done, cudaEventDisableTiming) == cudaSuccess;
-    }
+    ss.ok = cudaStreamCreateWithFlags(&ss.stream, cudaStreamNonBlocking) == cudaSuccess &&
+            cudaEventCreateWithFlags(&ss.fork, cudaEventDisableTiming) == cudaSuccess &&
+            cudaEventCreateWithFlags(&ss.done[0], cudaEventDisableTiming) == cudaSuccess &&
+            cudaEventCreateWithFlags(&ss.done[1], cudaEventDisableTiming) == cudaSuccess &&
+            cudaEventCreateWithFlags(&ss.bits_done, cudaEventDisableTiming) == cudaSuccess;
   }
   return ss;
 }
@@ -404,7 +396,6 @@ static int flush_wgrads(Ctx& c) {
   c.wgrad_done(ws);
   return 0;
 }
-static bool late_flush() { static const bool v = getenv("B200ST_LATE_FLUSH") != nullptr; return v; }
 struct WgradBlock {          // scope of one backward block: defers linear_wgrad launches until flush()
   Ctx& c;
   explicit WgradBlock(Ctx& cc) : c(cc) { c.defer_wgrads = true; }
@@ -596,7 +587,7 @@ static int self_attn_block_bwd(Ctx& c, const std::string& pre, const float* dx_o
   B200ST_TRY(attention_bwd(c, sv.dims, q, k, v, sv.p_pre, sv.p_drop, c.drop(cf.attention_dropout, sv.s_attn), sc.dctx, sc.S, sc.dS,
                            dq, dk, dv, sv.ctx, sv.lse, sv.bias, sv.causal, sc.dq32));
   B200ST_TRY(linear_wgrad(c, sv.h, d, sc.dqkv, 3 * d, M, d, 3 * d, pre + ".qkv.kernel", pre + ".qkv.bias"));
-  if (!late_flush()) B200ST_TRY(wb.flush());      // every dY of the block exists: the side stream starts under the rest of the chain
+  B200ST_TRY(wb.flush());      // every dY of the block exists: the side stream starts under the rest of the chain
   B200ST_TRY(linear_dgrad(c, sc.dqkv, 3 * d, M, 3 * d, d, pre + ".qkv.kernel", e0, sc.dh, F32, d));
   B200ST_TRY(block_ln_bwd(c, sc, sc.dh, sv.x_in, sv.mean, sv.rstd, pre, dx_out, dx_in, M, d));
   return wb.flush();
@@ -653,7 +644,7 @@ static int cross_attn_block_bwd(Ctx& c, const std::string& pre, const float* dx_
                            dq, dk, dv, sv.ctx, sv.lse, sv.bias, 0, sc.dq32));
   B200ST_TRY(linear_wgrad(c, sv.h, d, sc.dqkv, d, M, d, d, pre + ".q.kernel", pre + ".q.bias"));
   B200ST_TRY(linear_wgrad(c, sv.mem, d, sc.dkv, 2 * d, Mk, d, 2 * d, pre + ".kv.kernel", pre + ".kv.bias"));
-  if (!late_flush()) B200ST_TRY(wb.flush());
+  B200ST_TRY(wb.flush());
   B200ST_TRY(linear_dgrad(c, sc.dqkv, d, M, d, d, pre + ".q.kernel", e0, sc.dh, F32, d));
   B200ST_TRY(block_ln_bwd(c, sc, sc.dh, sv.x_in, sv.mean, sv.rstd, pre, dx_out, dx_in, M, d));
   GemmEpilogue ea = gemm_defaults().epi;
@@ -704,7 +695,7 @@ static int ffn_block_bwd(Ctx& c, const std::string& pre, const float* dx_out, fl
   if (c.dy_ready) c.dy_ready = false;      // produced by the previous block's LayerNorm-backward
   else RUN(cast_dropout(dx_out, sc.dY, c.adt, (int64_t)M * d, c.drop(cf.postprocess_dropout, sv.s_post), c.st));
   B200ST_TRY(linear_wgrad(c, sv.f1, f, sc.dY, d, M, f, d, pre + ".w2", pre + ".b2"));
-  if (fused_mlp_supported(M, d, f, c.adt) && !c.m.cfg.disable_fused_attention && !getenv("B200ST_NO_FUSED_MLP_BWD")) {
+  if (fused_mlp_supported(M, d, f, c.adt) && !c.m.cfg.disable_fused_attention) {
     // data-gradient chain in one kernel: dF1 = (dY W2^T) * relu'/dropout' (written for the W1 weight gradient), dh = dF1 W1^T
     const DropoutSpec fd = c.drop(cf.ffn_dropout, sv.s_ffn);
     RUN(cudaMemsetAsync(sc.dh, 0, sizeof(float) * (size_t)M * d, c.st) == cudaSuccess ? 0 : 1);
@@ -712,7 +703,7 @@ static int ffn_block_bwd(Ctx& c, const std::string& pre, const float* dx_out, fl
     RUN(fused_mlp_bwd(sc.dY, c.adt, M, d, f, c.W(pre + ".w1", 0, f).ptr, c.W(pre + ".w2", 0, d).ptr, sv.f1,
                       fd.p > 0.f ? fd.scale : 1.f, sc.dF1, sc.dh, c.st, tk));
     B200ST_TRY(linear_wgrad(c, sv.h, d, sc.dF1, f, M, d, f, pre + ".w1", pre + ".b1"));
-    if (!late_flush()) B200ST_TRY(wb.flush());
+    B200ST_TRY(wb.flush());
     B200ST_TRY(block_ln_bwd(c, sc, sc.dh, sv.x_in, sv.mean, sv.rstd, pre, dx_out, dx_in, M, d));
     return wb.flush();
   }
@@ -926,7 +917,7 @@ static int speech_front_bwd(Ctx& c, const float* src, const float* dx0, const Fr
   void* dz2 = c.act(R2 * C);
   // conv2's data gradient: implicit GEMMs straight from dz2 into class-major tiles (no [rows, 9C] column gradient), or the
   // explicit dcol = dz2 W^T + gather in conv1's backward
-  const bool implicit_dgrad = front_saves_xhat(cf) && is16(c.adt) && C == 256 && sv.F2 <= 128 && !getenv("B200ST_NO_IMPLICIT_DGRAD");
+  const bool implicit_dgrad = front_saves_xhat(cf) && is16(c.adt) && C == 256 && sv.F2 <= 128;
   void* dcol = c.act(implicit_dgrad ? conv2_dgrad_implicit_elems(B, sv.T2, sv.F2, C) : R2 * 9 * C);
   void* dz1 = c.act(R1 * C);
   const int K1p = (9 * cf.in_channels + 7) / 8 * 8;
@@ -1046,7 +1037,7 @@ static int model_run(Ctx& c, const Batch& b, bool backward) {
     comm_begin_step(c.sync);
     // the persistent GEMM grids assign tiles statically to `gridDim.x` CTAs: size them to the SMs NCCL leaves free, or the
     // CTAs that find no SM run as a second wave after the others have finished
-    if (comm_reserved_sms(c.sync) > 0) tc_debug().reserve_sms = comm_reserved_sms(c.sync);
+    gemm_set_reserved_sms(comm_reserved_sms(c.sync));
   }
   // reverse-arena-order buckets only when no tensor receives gradient later than its bucket (text models may tie the
   // source and target embeddings: one all-reduce at the end)
@@ -1100,7 +1091,7 @@ static int model_run(Ctx& c, const Batch& b, bool backward) {
   }
   c.join_side();        // the optimizer / all-reduce on `st` must see every weight gradient
   if (c.sync) {
-    tc_debug().reserve_sms = 0;
+    gemm_set_reserved_sms(0);
     B200ST_TRY(c.reduce_down_to(""));        // the rest (front-end, or everything when not bucketed)
     B200ST_TRY(comm_join(c.sync, c.st));
   }

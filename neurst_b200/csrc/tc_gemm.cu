@@ -56,8 +56,6 @@ struct TcParams {
   int conv_kpc;         // k-blocks per tap (C / 64)
   int conv_dt[4], conv_df[4], conv_wrow[4];   // per tap: time / frequency shift into dY, first row of the tap in the weight matrix
   uint32_t conv_a_bytes;                      // bytes one A box delivers (64 ch x conv_v x conv_tu x 2)
-  long long* dbg_trace; // perf experiments only: [cta][tile][8] clock64 stamps
-  int dbg_epi;          // perf experiments only (B200ST_EPI_MODE): 1 = no TMA store, 2 = no smem staging either, 3 = no TMEM read
 };
 
 struct TileCoord { int b2, b1, m_blk, n_blk, split; };
@@ -244,10 +242,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const TileCoord t = decode_tile(p, tile);
         const int kb0 = t.split * p.kb_per_split;
         const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-        int tix = (int)((tile - blockIdx.x) / gridDim.x);
         for (int kb = kb0; kb < kb1; ++kb) {
           ptx::mbar_wait(empty_bar(stage), phase ^ 1u);
-          if (p.dbg_trace && kb == kb0 && tix < 8) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 0] = clock64();
           const uint32_t sa = smem_base + stage * kStageBytes;
           const uint32_t sb = sa + kABytes;
           if constexpr (!A_MN && !B_MN) {
@@ -289,16 +285,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const TileCoord t = decode_tile(p, tile);
         const int kb0 = t.split * p.kb_per_split;
         const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-        int tix = (int)((tile - blockIdx.x) / gridDim.x);
-        if (p.dbg_trace && tix < 8) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 1] = clock64();
         ptx::mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
         ptx::tc_fence_after();
-        if (p.dbg_trace && tix < 8) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 2] = clock64();
         const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
         for (int kb = kb0; kb < kb1; ++kb) {
           ptx::mbar_wait(full_bar(stage), phase);
           ptx::tc_fence_after();
-          if (p.dbg_trace && tix < 8 && kb == kb0) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 3] = clock64();
           const uint32_t sa = smem_base + stage * kStageBytes;
           const uint32_t sb = sa + kABytes;
 #pragma unroll
@@ -311,7 +303,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           if (++stage == stages) { stage = 0; phase ^= 1u; }
         }
         ptx::mma_commit(tfull_bar(acc));         // accumulator ready for the epilogue warps
-        if (p.dbg_trace && tix < 8) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 4] = clock64();
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
       }
     }
@@ -326,11 +317,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const float relu_floor = ep.relu ? 0.f : -INFINITY;
     for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
       const TileCoord t = decode_tile(p, tile);
-      const int tix = (int)((tile - blockIdx.x) / gridDim.x);
-      if (p.dbg_trace && tix < 8 && warp == 2 && lane == 0) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 5] = clock64();
       ptx::mbar_wait(tfull_bar(acc), acc_phase);
       ptx::tc_fence_after();
-      if (p.dbg_trace && tix < 8 && warp == 2 && lane == 0) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 6] = clock64();
       const int m = t.m_blk * BM + row_in_tile;
       const int64_t bidx = (int64_t)t.b2 * p.nb1 + t.b1;
       const int64_t boff_c = (int64_t)t.b2 * p.c_sb2 + (int64_t)t.b1 * p.c_sb1;
@@ -366,27 +354,15 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           for (int cb = 0; cb < kColsPerBox / 32; ++cb) {
             const int co = c_begin_box + bx * kColsPerBox + cb * 32;
             uint32_t r[32];
-            if (p.dbg_epi >= 3) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j) r[j] = (uint32_t)(co + j);
-            } else {
-              ptx::tmem_ld_32x32b_x32(taddr_row + (uint32_t)co, r);
-              ptx::tmem_ld_wait();
-            }
+            ptx::tmem_ld_32x32b_x32(taddr_row + (uint32_t)co, r);
+            ptx::tmem_ld_wait();
             float v[32];
             epilogue_math<OUT>(p, r, er, co, relu_floor, v);
-            if (p.dbg_epi >= 2) {
-              float sacc = 0.f;
-#pragma unroll
-              for (int j = 0; j < 32; ++j) sacc += v[j];
-              if (sacc == 1.2345e-30f) stage_chunk<OUT>(buf, lane, cb, v);     // keeps the math alive, never taken
-            } else {
-              stage_chunk<OUT>(buf, lane, cb, v);
-            }
+            stage_chunk<OUT>(buf, lane, cb, v);
           }
           ptx::fence_proxy_async_smem();
           __syncwarp();
-          if (lane == 0 && p.dbg_epi == 0) {
+          if (lane == 0) {
             const int cn = n_base + c_begin_box + bx * kColsPerBox, cm = t.m_blk * BM + quad * 32;
             if (p.c_reduce)
               asm volatile("cp.reduce.async.bulk.tensor.4d.global.shared::cta.add.tile.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
@@ -416,7 +392,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       }
       ptx::tc_fence_before();
       __syncwarp();
-      if (p.dbg_trace && tix < 8 && warp == 2 && lane == 0) p.dbg_trace[((int64_t)blockIdx.x * 8 + tix) * 8 + 7] = clock64();
       if (lane == 0) ptx::mbar_arrive(tempty_bar(acc));
       if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
     }
@@ -1088,7 +1063,20 @@ int make_out_map(const void* C, int c_dtype, int N, int M, int nb1, int nb2, int
 }
 
 int g_num_sms = 0;
+int g_reserved_sms = 0;
 int64_t g_launches = 0;
+
+// SMs a persistent grid may occupy: the device's SMs less those reserved for concurrent communication kernels (a
+// reservation that would leave none is ignored)
+int usable_sms(int* out) {
+  if (g_num_sms == 0) {
+    int dev = 0;
+    B200ST_CUDA(cudaGetDevice(&dev));
+    B200ST_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
+  }
+  *out = g_reserved_sms > 0 && g_reserved_sms < g_num_sms ? g_num_sms - g_reserved_sms : g_num_sms;
+  return 0;
+}
 }  // namespace
 
 // 16-bit 4-D tensor map (inner, rows, nb1, nb2) with a {box_inner<=64, box_rows} box, 128B swizzle.
@@ -1149,10 +1137,7 @@ int launch_bn(bool a_mn, bool b_mn, const CUtensorMap& ta, const CUtensorMap& tb
 
 }  // namespace
 
-TcDebug& tc_debug() {
-  static TcDebug d{};
-  return d;
-}
+void gemm_set_reserved_sms(int n) { g_reserved_sms = n; }
 int64_t tc_launch_count() { return g_launches; }
 
 namespace {
@@ -1171,13 +1156,8 @@ int gemm_tc_impl(const GemmArgs& g, cudaStream_t stream, const ConvA* conv) {
     const bool wgrad = g.A.mn_major && g.B.mn_major;
     if ((wgrad && (abl & ABL_WGRAD)) || (!wgrad && (abl & ABL_GEMM))) return 0;
   }
-  if (g_num_sms == 0) {
-    int dev = 0;
-    B200ST_CUDA(cudaGetDevice(&dev));
-    B200ST_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
-  const TcDebug& dbg = tc_debug();
-  const int num_sms = dbg.max_ctas > 0 ? dbg.max_ctas : (dbg.reserve_sms > 0 && dbg.reserve_sms < g_num_sms ? g_num_sms - dbg.reserve_sms : g_num_sms);
+  int num_sms = 0;
+  B200ST_TRY(usable_sms(&num_sms));
 
   TcParams p{};
   p.M = g.M; p.N = g.N; p.K = g.K; p.nb1 = g.nb1; p.nb2 = g.nb2;
@@ -1193,15 +1173,14 @@ int gemm_tc_impl(const GemmArgs& g, cudaStream_t stream, const ConvA* conv) {
   const bool linear_epi = !g.epi.relu && !g.epi.mask_src && g.epi.drop.p == 0.f && !g.epi.residual && !g.epi.bias;
   const bool split_ok = linear_epi && g.c_dtype == F32 && g.epi.accumulate;
   if (g.splitk > 1) B200ST_CHECK(split_ok, "split-K needs a linear fp32 accumulate epilogue");
-  int bn = dbg.force_bn, splitk = g.splitk >= 1 ? g.splitk : 1;
+  int bn, splitk = g.splitk >= 1 ? g.splitk : 1;
   {
     double best = 1e30;
     int best_bn = 0, best_sk = 1;
     const int cands[3] = {256, 128, 64};
     for (int c : cands) {
-      if (dbg.force_bn && c != dbg.force_bn) continue;
       if (conv && c != 256) continue;
-      if (!dbg.force_bn && c > 64 && c >= 2 * ((g.N + 63) / 64 * 64)) continue;   // do not pad N by 2x or more
+      if (c > 64 && c >= 2 * ((g.N + 63) / 64 * 64)) continue;   // do not pad N by 2x or more
       const int64_t tiles0 = batch * p.m_tiles * ceil_div(g.N, c);
       int sk_lo = splitk, sk_hi = splitk;
       if (g.splitk == 0 && split_ok) {
@@ -1231,25 +1210,22 @@ int gemm_tc_impl(const GemmArgs& g, cudaStream_t stream, const ConvA* conv) {
   splitk = ceil_div(p.kb_total, p.kb_per_split);   // no empty trailing split
   p.splitk = splitk;
   p.atomic = (splitk > 1) ? 1 : 0;
-  p.dbg_epi = getenv("B200ST_EPI_MODE") ? atoi(getenv("B200ST_EPI_MODE")) : 0;
-  p.dbg_trace = getenv("B200ST_DEBUG_TRACE_PTR") ? reinterpret_cast<long long*>(strtoull(getenv("B200ST_DEBUG_TRACE_PTR"), nullptr, 0)) : nullptr;
   p.n_tiles = ceil_div(g.N, bn);
   p.num_tiles = batch * p.m_tiles * p.n_tiles * splitk;
 
+  // one CTA per SM (two co-resident CTAs were measured: no gain, see profiles/r01_gemm_notes.md)
   const uint32_t stage_bytes = kABytes + (uint32_t)bn * BK * 2;
-  const int ctas_per_sm = 1;   // (two co-resident CTAs per SM were measured: no gain, see profiles/r01_gemm_notes.md)
-  const int smem_budget = (ctas_per_sm == 2 ? (kSmemLimit / 2 - 1024) : kSmemLimit) - (int)kStagingBytes;
-  int stages = dbg.force_stages > 0 ? dbg.force_stages : (int)((smem_budget - 2048) / stage_bytes);
+  int stages = (int)((kSmemLimit - (int)kStagingBytes - 2048) / stage_bytes);
   if (stages > 8) stages = 8;
   p.stages = stages;
   const size_t smem = 1024 + (size_t)stages * stage_bytes + kStagingBytes + 8 * (2 * stages + 5) + 16;
   B200ST_CHECK(smem <= (size_t)kSmemLimit, "smem budget exceeded");
 
   // descriptors
-  const uint32_t mn_lbo = dbg.mn_lbo_bytes ? dbg.mn_lbo_bytes : 64u * BK * 2;   // next 64-wide MN chunk (TMA box)
-  const uint32_t mn_sbo = dbg.mn_sbo_bytes ? dbg.mn_sbo_bytes : 1024u;          // next group of 8 k-rows
-  const uint32_t k_lbo = dbg.k_lbo_bytes ? dbg.k_lbo_bytes : 16u;               // ignored for swizzled K-major
-  const uint32_t k_sbo = dbg.k_sbo_bytes ? dbg.k_sbo_bytes : 1024u;             // next group of 8 rows
+  const uint32_t mn_lbo = 64u * BK * 2;   // next 64-wide MN chunk (TMA box)
+  const uint32_t mn_sbo = 1024u;          // next group of 8 k-rows
+  const uint32_t k_lbo = 16u;             // ignored for swizzled K-major
+  const uint32_t k_sbo = 1024u;           // next group of 8 rows
   p.a_lbo = g.A.mn_major ? mn_lbo : k_lbo;  p.a_sbo = g.A.mn_major ? mn_sbo : k_sbo;
   p.b_lbo = g.B.mn_major ? mn_lbo : k_lbo;  p.b_sbo = g.B.mn_major ? mn_sbo : k_sbo;
   p.a_kstep = g.A.mn_major ? 16u * 128u : 32u;
@@ -1274,7 +1250,6 @@ int gemm_tc_impl(const GemmArgs& g, cudaStream_t stream, const ConvA* conv) {
   if (g.epi.residual)
     tma_ok = tma_ok && al16(g.epi.residual) && (g.epi.res_ld * 4) % 16 == 0 && (g.epi.res_sb1 * 4) % 16 == 0 && (g.epi.res_sb2 * 4) % 16 == 0;
   if (g.epi.drop.p > 0.f) tma_ok = tma_ok && g.epi.drop.bits != nullptr && (g.N % 32 == 0);
-  if (getenv("B200ST_NO_TMA_STORE")) tma_ok = false;
   p.use_tma_store = tma_ok ? 1 : 0;
   p.c_reduce = (p.atomic || g.epi.accumulate) ? 1 : 0;
   CUtensorMap tc;
@@ -1308,8 +1283,7 @@ int gemm_tc_impl(const GemmArgs& g, cudaStream_t stream, const ConvA* conv) {
     B200ST_TRY(make_operand_map(g.B, g.N, g.K, g.nb1, g.nb2, bn, &tb));
   }
 
-  const int max_grid = num_sms * ctas_per_sm;
-  const int grid = (int)(p.num_tiles < max_grid ? p.num_tiles : max_grid);
+  const int grid = (int)(p.num_tiles < num_sms ? p.num_tiles : num_sms);
   ++g_launches;
   if (g_prof) {
     ProfRec r{g, stream, bn, splitk};
@@ -1373,7 +1347,7 @@ int64_t conv2_dgrad_implicit_elems(int B, int T2, int F2, int C) {
 // fp32-accumulate MN-major x MN-major 16-bit GEMM with M % 128 == 0 and N % 256 == 0; returns 2 (nothing launched) when the
 // group does not qualify, so that the caller issues the products one by one.
 int gemm_wgrad_group(const GemmArgs* gs, int n, cudaStream_t stream) {
-  if (n < 2 || n > kMaxGroup || getenv("B200ST_NO_GROUPED_WGRAD")) return 2;
+  if (n < 2 || n > kMaxGroup) return 2;
   for (int i = 0; i < n; ++i) {
     const GemmArgs& g = gs[i];
     const bool plain = !g.epi.relu && !g.epi.mask_src && g.epi.drop.p == 0.f && !g.epi.residual && !g.epi.bias && g.epi.accumulate;
@@ -1383,13 +1357,8 @@ int gemm_wgrad_group(const GemmArgs* gs, int n, cudaStream_t stream) {
       return 2;
   }
   if (ablate_mask() & ABL_WGRAD) return 0;
-  if (g_num_sms == 0) {
-    int dev = 0;
-    B200ST_CUDA(cudaGetDevice(&dev));
-    B200ST_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
-  const TcDebug& dbg = tc_debug();
-  const int num_sms = dbg.max_ctas > 0 ? dbg.max_ctas : (dbg.reserve_sms > 0 && dbg.reserve_sms < g_num_sms ? g_num_sms - dbg.reserve_sms : g_num_sms);
+  int num_sms = 0;
+  B200ST_TRY(usable_sms(&num_sms));
   TcGroup grp;
   std::memset(&grp, 0, sizeof(grp));
   grp.n = n;
@@ -1452,25 +1421,29 @@ int gemm_wgrad_group(const GemmArgs* gs, int n, cudaStream_t stream) {
 // Fused FFN forward (see fused_mlp_fwd_kernel).  X: 16-bit [M, d] (LayerNorm output); W1 [d, ffn], W2 [ffn, d] in the same
 // 16-bit type (TF layouts); F1 out [M, ffn] (saved for the backward pass); x_out fp32 [M, d] must already hold the residual.
 bool fused_mlp_supported(int M, int d, int ffn, int dtype) {
-  return is16(dtype) && (d == 128 || d == 256) && ffn % 128 == 0 && M > 0 && !getenv("B200ST_NO_FUSED_MLP");
+  return is16(dtype) && (d == 128 || d == 256) && ffn % 128 == 0 && M > 0;
 }
+namespace {
+// slices of the hidden dimension: the most CTAs that still fit one wave, with an equal number of 128-column chunks per slice
+int mlp_splits(int M, int ffn, int* splits) {
+  int num_sms = 0;
+  B200ST_TRY(usable_sms(&num_sms));
+  const int m_tiles = ceil_div(M, BM), chunks = ffn / 128;
+  *splits = 1;
+  for (int s = 1; s <= chunks; ++s)
+    if (chunks % s == 0 && (int64_t)m_tiles * s <= num_sms) *splits = s;
+  return 0;
+}
+}  // namespace
 int fused_mlp_fwd(const void* X, int dtype, int M, int d, int ffn, const void* W1, const float* b1, const void* W2, const float* b2,
                   DropoutSpec drop_ffn, DropoutSpec drop_post, void* F1, float* x_out, cudaStream_t stream, int* tickets) {
   if (ablate_mask() & ABL_MLP_FWD) return 0;
   B200ST_CHECK(fused_mlp_supported(M, d, ffn, dtype), "fused MLP: unsupported shape / dtype");
-  if (g_num_sms == 0) {
-    int dev = 0;
-    B200ST_CUDA(cudaGetDevice(&dev));
-    B200ST_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
   if (drop_ffn.p > 0.f) B200ST_CHECK(drop_ffn.bits != nullptr, "fused MLP needs precomputed dropout bits");
   if (drop_post.p > 0.f) B200ST_CHECK(drop_post.bits != nullptr, "fused MLP needs precomputed dropout bits");
   const int m_tiles = ceil_div(M, BM), chunks = ffn / 128;
-  // slices of the hidden dimension: the most CTAs that still fit one wave, with an equal number of chunks per slice
   int splits = 1;
-  for (int s2 = 1; s2 <= chunks; ++s2)
-    if (chunks % s2 == 0 && (int64_t)m_tiles * s2 <= g_num_sms - tc_debug().reserve_sms) splits = s2;
-  if (getenv("B200ST_MLP_SPLITS")) { const int f = atoi(getenv("B200ST_MLP_SPLITS")); if (f >= 1 && chunks % f == 0) splits = f; }
+  B200ST_TRY(mlp_splits(M, ffn, &splits));
   MlpParams p{};
   p.M = M; p.d = d; p.ffn = ffn; p.splits = splits; p.chunks_per_cta = chunks / splits;
   p.b1 = b1; p.b2 = b2; p.drop_ffn = drop_ffn; p.drop_post = drop_post;
@@ -1501,16 +1474,9 @@ int fused_mlp_bwd(const void* dY, int dtype, int M, int d, int ffn, const void* 
                   void* dF1, float* dH, cudaStream_t stream, int* tickets) {
   if (ablate_mask() & ABL_MLP_BWD) return 0;
   B200ST_CHECK(fused_mlp_supported(M, d, ffn, dtype), "fused MLP: unsupported shape / dtype");
-  if (g_num_sms == 0) {
-    int dev = 0;
-    B200ST_CUDA(cudaGetDevice(&dev));
-    B200ST_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
   const int m_tiles = ceil_div(M, BM), chunks = ffn / 128;
   int splits = 1;
-  for (int s2 = 1; s2 <= chunks; ++s2)
-    if (chunks % s2 == 0 && (int64_t)m_tiles * s2 <= g_num_sms - tc_debug().reserve_sms) splits = s2;
-  if (getenv("B200ST_MLP_SPLITS")) { const int f = atoi(getenv("B200ST_MLP_SPLITS")); if (f >= 1 && chunks % f == 0) splits = f; }
+  B200ST_TRY(mlp_splits(M, ffn, &splits));
   MlpParams p{};
   p.M = M; p.d = d; p.ffn = ffn; p.splits = splits; p.chunks_per_cta = chunks / splits;
   p.b1 = nullptr; p.b2 = nullptr; p.drop_ffn = no_dropout(); p.drop_post = no_dropout();

@@ -206,7 +206,7 @@ class GreedyArgs(C.Structure):
 
 # every symbol include/b200st.h declares (tests/test_abi.py checks the .so exports all of them)
 EXPORTS = [
-    "b200st_last_error", "b200st_version", "b200st_launch_count", "b200st_gemm", "b200st_gemm_bench", "b200st_debug_tc", "b200st_profile_begin", "b200st_profile_end",
+    "b200st_last_error", "b200st_version", "b200st_launch_count", "b200st_gemm", "b200st_gemm_bench", "b200st_profile_begin", "b200st_profile_end",
     "b200st_create", "b200st_destroy", "b200st_param_arena_numel", "b200st_param_count", "b200st_param_info",
     "b200st_workspace_bytes", "b200st_forward", "b200st_forward_backward", "b200st_refresh_shadow", "b200st_adam_step", "b200st_optimizer_step",
     "b200st_comm_unique_id", "b200st_comm_init", "b200st_comm_broadcast", "b200st_comm_destroy", "b200st_comm_stats", "b200st_train_step",

@@ -22,6 +22,19 @@ def test_library_exports_every_declared_symbol():
     assert lib.b200st_version() == L.ABI_VERSION
 
 
+def test_library_reads_only_measurement_environment_variables():
+    """Environment variables may switch on measurement (ablation, PDL off for per-kernel attribution, the GEMM profile
+    CSV) or cap NCCL's CTAs, never choose between implementations: every other path would be untested."""
+    csrc = os.path.join(ROOT, "neurst_b200", "csrc")
+    args = []
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh", ".c")):
+            args += re.findall(r"\bgetenv\(\s*([^)]*?)\s*\)", open(os.path.join(csrc, f)).read())
+    names = {a[1:-1] for a in args if re.fullmatch(r'"[^"]+"', a)}
+    assert len(names) == len(set(args)), "getenv with a non-literal name: %s" % args
+    assert names == {"B200ST_ABLATE", "B200ST_NO_PDL", "B200ST_PROFILE_CSV", "B200ST_NCCL_MAX_CTAS"}
+
+
 def test_io_library_exports_every_declared_symbol():
     import ctypes
     from neurst_b200.csrc import build as B

@@ -24,6 +24,3 @@ B200ST_NO_PDL=1 timeout 200 ncu --set full --clock-control none --import-source 
 B200ST_NO_PDL=1 timeout 200 ncu --set full --clock-control none --import-source on -k regex:fused_mlp_fwd_kernel -s 10 -c 1 -f -o $O/r02_final_fused_mlp \
   python tools/one_step.py 1 > $O/r02_final_ncu_mlp.log 2>&1; tail -1 $O/r02_final_ncu_mlp.log | cut -c1-160
 ls -la $O/r02_final_* | cut -c30-200
-echo "== A/B: conv1 forward with packed fp32x2 FMAs"
-(B200ST_CONV1_FFMA2=1 timeout 200 python -m pytest tests/test_model_gpu.py -q -k "oracle or fixture" 2>&1 | tail -2)
-(B200ST_CONV1_FFMA2=1 timeout 150 python bench.py --steps 20 --warmup 5 --no-cpu-baseline 2>>$O/r02_final_bench.err | tail -1) > $O/r02_final_bench_cfg2_ffma2.json; cut -c1-200 $O/r02_final_bench_cfg2_ffma2.json
