@@ -252,6 +252,32 @@ int b200st_conv1_ln_relu_fwd(const float* src, const float* w, const float* b, c
 uint64_t b200st_dropout_stream_id(const char* site);
 int b200st_dropout_mask(uint64_t seed, uint64_t stream_id, int64_t n, float p, uint8_t* out, void* stream);
 
+/* tests only: the fused 16-bit attention and FFN kernels called on their own (dt = 1 bf16, 2 fp16).
+ * Dropout is a probability plus a caller-owned keep bitmap: byte g holds the keep bits of elements 8g .. 8g+7 (bit j =
+ * element 8g+j, the packing of b200st_dropout_mask); a bitmap is required when p > 0.
+ * Attention (head dim 64): q/k/v/ctx/dq/dk/dv are [B*T, ld] row views, head h at columns [64h, 64h+64); bias [B, Tk]
+ * additive or NULL; kv_len [B] or NULL (keys >= kv_len[b] carry the -1e9 bias: whole key blocks past it are skipped);
+ * keep_bits [B, H, Tq, round8(Tk)]; lse [B, H, Tq] (natural log); dq_scratch fp32 with B*Tq*H*64 + B*H*Tq elements. */
+int b200st_attention_fwd(int32_t dt, const void* q, int64_t q_ld, const void* k, int64_t k_ld, const void* v, int64_t v_ld,
+                         int32_t B, int32_t H, int32_t Tq, int32_t Tk, const float* bias, const int32_t* kv_len,
+                         int32_t causal, float drop_p, const uint8_t* keep_bits, void* ctx, int64_t ctx_ld, float* lse,
+                         void* stream);
+int b200st_attention_bwd(int32_t dt, const void* q, int64_t q_ld, const void* k, int64_t k_ld, const void* v, int64_t v_ld,
+                         int32_t B, int32_t H, int32_t Tq, int32_t Tk, const float* bias, const int32_t* kv_len,
+                         int32_t causal, float drop_p, const uint8_t* keep_bits, const void* ctx, int64_t ctx_ld,
+                         const void* dctx, int64_t dctx_ld, const float* lse, float* dq_scratch, void* dq, int64_t dq_ld,
+                         void* dk, int64_t dk_ld, void* dv, int64_t dv_ld, void* stream);
+/* FFN (d in {128, 256}, ffn % 128 == 0), all row-major and packed: X [M, d], W1 [d, ffn], W2 [ffn, d] in dt; b1 [ffn],
+ * b2 [d] fp32 or NULL; ffn_bits [M, ffn], post_bits [M, d].  Forward: F1 = dropout(relu(X W1 + b1)) [M, ffn] in dt,
+ * x_out [M, d] fp32 += post-dropout(F1 W2 + b2).  Backward: dF1 = scale * (dY W2^T) where F1 > 0 [M, ffn] in dt,
+ * dH [M, d] fp32 += dF1 W1^T.  tickets: NULL, or int [ceil(M / 128)] all zero (slices then add in a fixed order; the
+ * kernel leaves them zero).  splits_out (may be NULL): the number of hidden slices the launch used. */
+int b200st_ffn_fwd(int32_t dt, const void* X, int32_t M, int32_t d, int32_t ffn, const void* W1, const float* b1,
+                   const void* W2, const float* b2, float drop_ffn_p, const uint8_t* ffn_bits, float drop_post_p,
+                   const uint8_t* post_bits, void* F1, float* x_out, int32_t* tickets, int32_t* splits_out, void* stream);
+int b200st_ffn_bwd(int32_t dt, const void* dY, int32_t M, int32_t d, int32_t ffn, const void* W1, const void* W2,
+                   const void* F1, float scale, void* dF1, float* dH, int32_t* tickets, int32_t* splits_out, void* stream);
+
 /* tests/bench only: time `iters` back-to-back launches of one GEMM with CUDA events on `stream` (no host overhead) */
 int b200st_gemm_bench(const b200st_gemm_args* args, int32_t iters, float* ms_per_iter, void* stream);
 

@@ -80,34 +80,28 @@ __device__ __forceinline__ float ex2_approx(float x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-// 64 keep-bits (keys k0 .. k0+63 of one query row) from the precomputed bitmap or regenerated; bits of keys >= Tkp read as 1
-__device__ __forceinline__ void load_keep64(const DropoutSpec& d, bool row_ok, int64_t row_bit0, int k0, int Tkp, uint32_t thresh,
-                                            uint32_t (&keep)[2]) {
+// 64 keep-bits (keys k0 .. k0+63 of one query row) from the precomputed bitmap [B, H, Tq, Tkp] (the host refuses p > 0
+// without one); bits of keys >= Tkp read as 1
+__device__ __forceinline__ void load_keep64(const uint8_t* row_bits, int k0, int Tkp, uint32_t (&keep)[2]) {
   keep[0] = keep[1] = 0xffffffffu;
-  if (!(d.p > 0.f) || !row_ok) return;
-  if (d.bits && (Tkp & 63) == 0) {        // rows are 8-byte aligned in the bitmap: one 64-bit load
+  if (!row_bits) return;
+  if ((Tkp & 63) == 0) {                  // rows are 8-byte aligned in the bitmap: one 64-bit load
     if (k0 < Tkp) {
-      const uint2 w = __ldg(reinterpret_cast<const uint2*>(d.bits + ((uint64_t)(row_bit0 + k0) >> 3)));
+      const uint2 w = __ldg(reinterpret_cast<const uint2*>(row_bits + (k0 >> 3)));
       keep[0] = w.x; keep[1] = w.y;
     }
     return;
   }
-  if (d.bits) {                           // bitmap, unaligned rows: 8 byte loads (all issued before the first use)
-    uint32_t byte[8];
-    const uint8_t* bp = d.bits + ((uint64_t)(row_bit0 + k0) >> 3);
+  uint32_t byte[8];                       // unaligned rows: 8 byte loads (all issued before the first use)
+  const uint8_t* bp = row_bits + (k0 >> 3);
 #pragma unroll
-    for (int g = 0; g < 8; ++g) byte[g] = (k0 + 8 * g < Tkp) ? (uint32_t)__ldg(bp + g) : 0xffu;
-    keep[0] = byte[0] | (byte[1] << 8) | (byte[2] << 16) | (byte[3] << 24);
-    keep[1] = byte[4] | (byte[5] << 8) | (byte[6] << 16) | (byte[7] << 24);
-    return;
-  }
-#pragma unroll 1
-  for (int g = 0; g < 8; ++g) {           // no bitmap: regenerate with Philox (stand-alone attention API)
-    if (k0 + 8 * g < Tkp) {
-      const uint32_t byte = dropout_keep8(dropout_seed(d), d.stream, (uint64_t)(row_bit0 + k0 + 8 * g) >> 3, thresh);
-      keep[g >> 2] = (keep[g >> 2] & ~(0xffu << (8 * (g & 3)))) | (byte << (8 * (g & 3)));
-    }
-  }
+  for (int g = 0; g < 8; ++g) byte[g] = (k0 + 8 * g < Tkp) ? (uint32_t)__ldg(bp + g) : 0xffu;
+  keep[0] = byte[0] | (byte[1] << 8) | (byte[2] << 16) | (byte[3] << 24);
+  keep[1] = byte[4] | (byte[5] << 8) | (byte[6] << 16) | (byte[7] << 24);
+}
+// keep-bit row of (b, h, query row) in the bitmap, or null when the row takes no dropout
+__device__ __forceinline__ const uint8_t* keep_row(const AttnParams& p, bool row_ok, int64_t row_g) {
+  return (p.drop.p > 0.f && row_ok) ? p.drop.bits + row_g * (p.Tkp >> 3) : nullptr;
 }
 
 template <bool CAUSAL, int DT>
@@ -210,19 +204,20 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     const int q = qt * BQ + row;
     const int64_t row_g = ((int64_t)b * p.H + h) * p.Tq + q;
     const uint32_t lane_addr = (uint32_t)(quad * 32) << 16;
-    const uint32_t thresh = dropout_thresh16(p.drop.p);
     const float a2 = p.alpha * kLog2e;
     const int qlim = q + (p.Tk - p.Tq);               // causal: keys k > qlim get the additive FLOAT_MIN
     const float cmask = kMaskMin * kLog2e;
     {
       const float* bias_row = p.bias ? p.bias + (int64_t)b * p.Tk : nullptr;
+#pragma unroll 1          // unrolled, this one-off loop costs the causal instantiation extra spill slots
       for (int k = threadIdx.x - 64; k < nblk * BKV; k += 256)
         btab[k] = (k < p.Tk) ? (bias_row ? __ldg(bias_row + k) * kLog2e : 0.f) : -INFINITY;
       softmax_bar();
     }
     float m = -INFINITY, l = 0.f;      // running row max (log2 domain, shared by both halves) and this half's partial sum
     uint32_t keep[2], keep_next[2];
-    load_keep64(p.drop, q < p.Tq, row_g * p.Tkp, half * 64, p.Tkp, thresh, keep);
+    const uint8_t* krow = keep_row(p, q < p.Tq, row_g);
+    load_keep64(krow, half * 64, p.Tkp, keep);
     for (int j = 0; j < nblk; ++j) {
       const uint32_t ph = (uint32_t)j & 1u;
       const int kbase = j * BKV + half * 64;          // first key of this thread's 64 columns
@@ -236,7 +231,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         __syncwarp();
         ptx::tmem_ld_32x32b_x32(tS + lane_addr + half * 64, r0);
         ptx::tmem_ld_32x32b_x32(tS + lane_addr + half * 64 + 32, r1);
-        if (j + 1 < nblk) load_keep64(p.drop, q < p.Tq, row_g * p.Tkp, kbase + BKV, p.Tkp, thresh, keep_next);   // in flight during the math
+        if (j + 1 < nblk) load_keep64(krow, kbase + BKV, p.Tkp, keep_next);   // in flight during the math
         __syncwarp();
         ptx::tmem_ld_wait();
       }
@@ -469,7 +464,6 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     const int quarter = (warp - 2) >> 2;             // 0..3: key columns [32 * quarter, +32)
     const int row = quad * 32 + lane;
     const uint32_t lane_addr = (uint32_t)(quad * 32) << 16;
-    const uint32_t thresh = dropout_thresh16(p.drop.p);
     const float a2 = p.alpha * kLog2e;
     const float cmask = kMaskMin * kLog2e;
     const float dscale = (p.drop.p > 0.f) ? p.drop.scale : 1.0f;
@@ -487,24 +481,29 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     const float4* bt4 = reinterpret_cast<const float4*>(btab + c0);
     // per-tile row scalars (D = rowsum(dO * O), LSE in the log2 domain: +inf on padding rows => P = 0, keep bits) are
     // prefetched one tile ahead so their global-load latency hides behind the previous tile's math
-    auto load_row = [&](int i, float& Dq, float& lse2, uint32_t& keep) {
+    // A row whose every key carries the -1e9 bias (a length-0 sequence): in fp32 each logit the forward pass visited
+    // equals that bias (s is absorbed), so its softmax is uniform over those keys, but the stored LSE (-1e9) has absorbed
+    // log(l) as well and exp2(x - lse2) gives 1 for every key.  Such rows scale P by 1 / (keys the forward pass visited).
+    const int kv_vis = p.kv_len ? min(p.Tk, max(1, (__ldg(p.kv_len + b) + BKV - 1) / BKV) * BKV) : p.Tk;
+    auto load_row = [&](int i, float& Dq, float& lse2, float& prs, uint32_t& keep) {
       const int q = i * BQ + row;
       const bool qv = q < p.Tq;
       const int64_t row_g = ((int64_t)b * p.H + h) * p.Tq + q;
       Dq = qv ? __ldg(p.dvec + row_g) : 0.f;
       lse2 = qv ? __ldg(p.lse + row_g) * kLog2e : INFINITY;
+      prs = lse2 < 0.5f * cmask ? 1.f / (float)(CAUSAL ? min(kv_vis, q + (p.Tk - p.Tq) + 1) : kv_vis) : 1.f;
       uint32_t k2[2];
-      load_keep64(p.drop, qv, row_g * p.Tkp, kbase64, p.Tkp, thresh, k2);
+      load_keep64(keep_row(p, qv, row_g), kbase64, p.Tkp, k2);
       keep = k2[quarter & 1];
     };
-    float Dq, lse2, Dq_n = 0.f, lse2_n = INFINITY;
+    float Dq, lse2, prs, Dq_n = 0.f, lse2_n = INFINITY, prs_n = 1.f;
     uint32_t keep, keep_n = 0xffffffffu;
-    load_row(0, Dq, lse2, keep);
+    load_row(0, Dq, lse2, prs, keep);
     for (int i = 0; i < nq; ++i) {
       const int q = i * BQ + row;
       const bool qv = q < p.Tq;
       const int qlim = q + (p.Tk - p.Tq);
-      if (i + 1 < nq) load_row(i + 1, Dq_n, lse2_n, keep_n);
+      if (i + 1 < nq) load_row(i + 1, Dq_n, lse2_n, prs_n, keep_n);
       __syncwarp();
       ptx::mbar_wait(sdp_full, (uint32_t)i & 1u);
       ptx::tc_fence_after();
@@ -524,7 +523,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
           for (int t = 0; t < 8; ++t) {
             float x = fmaf(__uint_as_float(rs[g8 * 8 + t]), a2, bb[t]);
             if (CAUSAL) x = (jb * BKV + c0 + g8 * 8 + t > qlim) ? x + cmask : x;
-            const float pr = ex2_approx(x - lse2);
+            const float pr = ex2_approx(x - lse2) * prs;
             const bool kp = (kb >> t) & 1u;
             const float dpv = kp ? __uint_as_float(rp[g8 * 8 + t]) : 0.f;
             pd[t] = kp ? pr : 0.f;
@@ -558,7 +557,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(dq_empty);
-      Dq = Dq_n; lse2 = lse2_n; keep = keep_n;
+      Dq = Dq_n; lse2 = lse2_n; prs = prs_n; keep = keep_n;
     }
     // ---- dV, dK of this kv block (all MMAs retired: the last dq_full commit covers them); 16 columns per warp ----
     const int kk = jb * BKV + row;
@@ -658,6 +657,7 @@ int attention_fwd_fused(int dt, const void* q, int64_t q_ld, const void* k, int6
   B200ST_CHECK(Tq > 0 && Tk > 0 && B > 0 && H > 0, "empty attention");
   B200ST_CHECK(B <= 65535 && H <= 65535, "attention grid too large");
   B200ST_CHECK(is16(dt), "fused attention needs a 16-bit operand type");
+  if (drop.p > 0.f) B200ST_CHECK(drop.bits != nullptr, "fused attention needs precomputed dropout bits");
   CUtensorMap tq, tk, tv;
   B200ST_TRY(make_tma_map_16(q, dt, DH, Tq, H, B, q_ld, DH, (int64_t)Tq * q_ld, BQ, &tq));
   B200ST_TRY(make_tma_map_16(k, dt, DH, Tk, H, B, k_ld, DH, (int64_t)Tk * k_ld, BKV, &tk));
@@ -694,6 +694,7 @@ int attention_bwd_fused(int dt, const void* q, int64_t q_ld, const void* k, int6
   if (ablate_mask() & ABL_ATTN_BWD) return 0;
   B200ST_CHECK(Tq > 0 && Tk > 0 && B > 0 && H > 0 && B <= 65535 && H <= 65535, "bad attention shape");
   B200ST_CHECK(is16(dt), "fused attention needs a 16-bit operand type");
+  if (drop.p > 0.f) B200ST_CHECK(drop.bits != nullptr, "fused attention needs precomputed dropout bits");
   CUtensorMap tq, tk, tv, tdo;
   B200ST_TRY(make_tma_map_16(q, dt, DH, Tq, H, B, q_ld, DH, (int64_t)Tq * q_ld, BQ, &tq));
   B200ST_TRY(make_tma_map_16(k, dt, DH, Tk, H, B, k_ld, DH, (int64_t)Tk * k_ld, BKV, &tk));

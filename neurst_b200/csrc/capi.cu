@@ -341,6 +341,54 @@ int b200st_conv1_ln_relu_fwd(const float* src, const float* w, const float* b, c
 
 uint64_t b200st_dropout_stream_id(const char* site) { return site ? dropout_stream_id(site) : 0; }
 
+// ---- the fused 16-bit kernels on their own (tests) ----
+static int test_dropout(float p, const uint8_t* bits, DropoutSpec* d) {
+  B200ST_CHECK(p >= 0.f && p < 1.f, "dropout probability must be in [0, 1)");
+  B200ST_CHECK(p == 0.f || bits != nullptr, "dropout p > 0 needs a keep bitmap");
+  *d = p > 0.f ? DropoutSpec{p, 1.f / (1.f - p), 0, 0, nullptr, bits} : no_dropout();
+  return 0;
+}
+int b200st_attention_fwd(int32_t dt, const void* q, int64_t q_ld, const void* k, int64_t k_ld, const void* v, int64_t v_ld,
+                         int32_t B, int32_t H, int32_t Tq, int32_t Tk, const float* bias, const int32_t* kv_len,
+                         int32_t causal, float drop_p, const uint8_t* keep_bits, void* ctx, int64_t ctx_ld, float* lse,
+                         void* stream) {
+  if (!q || !k || !v || !ctx || !lse) B200ST_FAIL("null argument");
+  B200ST_CHECK(is16(dt), "fused attention needs a 16-bit type (1 = bf16, 2 = fp16)");
+  DropoutSpec d;
+  B200ST_TRY(test_dropout(drop_p, keep_bits, &d));
+  return attention_fwd_fused(dt, q, q_ld, k, k_ld, v, v_ld, B, H, Tq, Tk, bias, causal, d, ctx, ctx_ld, lse,
+                             reinterpret_cast<cudaStream_t>(stream), kv_len);
+}
+int b200st_attention_bwd(int32_t dt, const void* q, int64_t q_ld, const void* k, int64_t k_ld, const void* v, int64_t v_ld,
+                         int32_t B, int32_t H, int32_t Tq, int32_t Tk, const float* bias, const int32_t* kv_len,
+                         int32_t causal, float drop_p, const uint8_t* keep_bits, const void* ctx, int64_t ctx_ld,
+                         const void* dctx, int64_t dctx_ld, const float* lse, float* dq_scratch, void* dq, int64_t dq_ld,
+                         void* dk, int64_t dk_ld, void* dv, int64_t dv_ld, void* stream) {
+  if (!q || !k || !v || !ctx || !dctx || !lse || !dq_scratch || !dq || !dk || !dv) B200ST_FAIL("null argument");
+  B200ST_CHECK(is16(dt), "fused attention needs a 16-bit type (1 = bf16, 2 = fp16)");
+  DropoutSpec d;
+  B200ST_TRY(test_dropout(drop_p, keep_bits, &d));
+  return attention_bwd_fused(dt, q, q_ld, k, k_ld, v, v_ld, ctx, ctx_ld, dctx, dctx_ld, lse, B, H, Tq, Tk, bias, causal, d,
+                             dq_scratch, dq, dq_ld, dk, dk_ld, dv, dv_ld, reinterpret_cast<cudaStream_t>(stream), kv_len);
+}
+int b200st_ffn_fwd(int32_t dt, const void* X, int32_t M, int32_t d, int32_t ffn, const void* W1, const float* b1,
+                   const void* W2, const float* b2, float drop_ffn_p, const uint8_t* ffn_bits, float drop_post_p,
+                   const uint8_t* post_bits, void* F1, float* x_out, int32_t* tickets, int32_t* splits_out, void* stream) {
+  if (!X || !W1 || !W2 || !F1 || !x_out) B200ST_FAIL("null argument");
+  B200ST_CHECK(fused_mlp_supported(M, d, ffn, dt), "fused FFN: needs a 16-bit type, d in {128, 256}, ffn % 128 == 0 and M > 0");
+  DropoutSpec d1, d2;
+  B200ST_TRY(test_dropout(drop_ffn_p, ffn_bits, &d1));
+  B200ST_TRY(test_dropout(drop_post_p, post_bits, &d2));
+  return fused_mlp_fwd(X, dt, M, d, ffn, W1, b1, W2, b2, d1, d2, F1, x_out, reinterpret_cast<cudaStream_t>(stream), tickets,
+                       splits_out);
+}
+int b200st_ffn_bwd(int32_t dt, const void* dY, int32_t M, int32_t d, int32_t ffn, const void* W1, const void* W2,
+                   const void* F1, float scale, void* dF1, float* dH, int32_t* tickets, int32_t* splits_out, void* stream) {
+  if (!dY || !W1 || !W2 || !F1 || !dF1 || !dH) B200ST_FAIL("null argument");
+  B200ST_CHECK(fused_mlp_supported(M, d, ffn, dt), "fused FFN: needs a 16-bit type, d in {128, 256}, ffn % 128 == 0 and M > 0");
+  return fused_mlp_bwd(dY, dt, M, d, ffn, W1, W2, F1, scale, dF1, dH, reinterpret_cast<cudaStream_t>(stream), tickets, splits_out);
+}
+
 }  // extern "C"
 
 namespace b200st {

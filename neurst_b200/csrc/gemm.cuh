@@ -79,11 +79,13 @@ int gemm(const GemmArgs& g, cudaStream_t stream);
 // (dropout(relu(X W1 + b1)) W2 + b2); the hidden activations are also written to F1 for the backward pass.
 bool fused_mlp_supported(int M, int d, int ffn, int dtype);
 int fused_mlp_fwd(const void* X, int dtype, int M, int d, int ffn, const void* W1, const float* b1, const void* W2, const float* b2,
-                  DropoutSpec drop_ffn, DropoutSpec drop_post, void* F1, float* x_out, cudaStream_t stream, int* tickets = nullptr);
+                  DropoutSpec drop_ffn, DropoutSpec drop_post, void* F1, float* x_out, cudaStream_t stream, int* tickets = nullptr,
+                  int* splits_out = nullptr);
 // tickets (optional): int [ceil(M / 128)], zero before the first use: hidden slices reduce in slice order (deterministic)
+// splits_out (optional): receives the number of hidden slices the launch used
 
 int fused_mlp_bwd(const void* dY, int dtype, int M, int d, int ffn, const void* W1, const void* W2, const void* F1, float scale,
-                  void* dF1, float* dH, cudaStream_t stream, int* tickets = nullptr);
+                  void* dF1, float* dH, cudaStream_t stream, int* tickets = nullptr, int* splits_out = nullptr);
 
 // SMs the persistent tcgen05 grids leave to concurrent communication kernels (set by the model while gradient all-reduces
 // overlap the backward pass; 0 = none)

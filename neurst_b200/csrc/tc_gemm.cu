@@ -1436,7 +1436,8 @@ int mlp_splits(int M, int ffn, int* splits) {
 }
 }  // namespace
 int fused_mlp_fwd(const void* X, int dtype, int M, int d, int ffn, const void* W1, const float* b1, const void* W2, const float* b2,
-                  DropoutSpec drop_ffn, DropoutSpec drop_post, void* F1, float* x_out, cudaStream_t stream, int* tickets) {
+                  DropoutSpec drop_ffn, DropoutSpec drop_post, void* F1, float* x_out, cudaStream_t stream, int* tickets,
+                  int* splits_out) {
   if (ablate_mask() & ABL_MLP_FWD) return 0;
   B200ST_CHECK(fused_mlp_supported(M, d, ffn, dtype), "fused MLP: unsupported shape / dtype");
   if (drop_ffn.p > 0.f) B200ST_CHECK(drop_ffn.bits != nullptr, "fused MLP needs precomputed dropout bits");
@@ -1465,13 +1466,14 @@ int fused_mlp_fwd(const void* X, int dtype, int M, int d, int ffn, const void* W
   launch_pdl(kern, m_tiles * splits, kThreads, kMlpSmem, stream, tx, tw1, tw2, tf1, tout, p);
   ++g_launches;
   B200ST_LAUNCH_CHECK();
+  if (splits_out) *splits_out = splits;
   return 0;
 }
 
 // Fused FFN backward, data-gradient chain: dF1 = scale * (dY W2^T) masked by (F1 > 0)  [written for the W1 weight gradient],
-// dH += dF1 W1^T (fp32, dH must be zero-initialised).  Same kernel, weights read as K-major B operands.
+// dH += dF1 W1^T (fp32 reduce-add into what dH holds; the model zero-initialises it).  Same kernel, weights read as K-major B operands.
 int fused_mlp_bwd(const void* dY, int dtype, int M, int d, int ffn, const void* W1, const void* W2, const void* F1, float scale,
-                  void* dF1, float* dH, cudaStream_t stream, int* tickets) {
+                  void* dF1, float* dH, cudaStream_t stream, int* tickets, int* splits_out) {
   if (ablate_mask() & ABL_MLP_BWD) return 0;
   B200ST_CHECK(fused_mlp_supported(M, d, ffn, dtype), "fused MLP: unsupported shape / dtype");
   const int m_tiles = ceil_div(M, BM), chunks = ffn / 128;
@@ -1498,6 +1500,7 @@ int fused_mlp_bwd(const void* dY, int dtype, int M, int d, int ffn, const void* 
   launch_pdl(kern, m_tiles * splits, kThreads, kMlpSmem, stream, tx, tw1, tw2, tf1, tout, p);
   ++g_launches;
   B200ST_LAUNCH_CHECK();
+  if (splits_out) *splits_out = splits;
   return 0;
 }
 

@@ -214,6 +214,7 @@ EXPORTS = [
     "b200st_greedy_search", "b200st_greedy_used_graph",
     "b200st_encoder_forward", "b200st_decoder_forward", "b200st_mha_forward", "b200st_lsce", "b200st_layernorm_fwd",
     "b200st_layernorm_bwd", "b200st_softmax_fwd", "b200st_conv1_ln_relu_fwd", "b200st_dropout_stream_id", "b200st_dropout_mask",
+    "b200st_attention_fwd", "b200st_attention_bwd", "b200st_ffn_fwd", "b200st_ffn_bwd",
 ]
 
 
@@ -268,6 +269,19 @@ def _declare(lib):
     lib.b200st_softmax_fwd.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int64,
                                        C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
     lib.b200st_dropout_mask.argtypes = [C.c_uint64, C.c_uint64, C.c_int64, C.c_float, C.c_void_p, C.c_void_p]
+    lib.b200st_attention_fwd.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                         C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                         C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+    lib.b200st_attention_bwd.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                         C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                         C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                         C.c_void_p]
+    lib.b200st_ffn_fwd.argtypes = [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_float, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]
+    lib.b200st_ffn_bwd.argtypes = [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]
     lib.b200st_gemm.argtypes = [C.POINTER(GemmArgs), C.c_void_p]
     lib.b200st_gemm_bench.argtypes = [C.POINTER(GemmArgs), C.c_int32, C.POINTER(C.c_float), C.c_void_p]
 
@@ -291,6 +305,79 @@ def layernorm(x, gamma, beta, eps, out_dtype=None, relu=False):
     check(load().b200st_layernorm_fwd(x.data_ptr(), _dt(x), gamma.data_ptr(), beta.data_ptr(), eps, y.data_ptr(), _dt(y),
                                       None, None, rows, cols, int(relu), _stream()))
     return y
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _rows(t, cols=None):
+    """(rows, row stride) of a 2-D row view with a unit inner stride (a column slice of a packed buffer is fine)."""
+    assert t.dim() == 2 and t.stride(1) == 1, "expected a 2-D view with a contiguous inner dimension"
+    assert cols is None or t.shape[1] == cols, (tuple(t.shape), cols)
+    return t.shape[0], t.stride(0)
+
+
+def attention_fwd(q, k, v, ctx, lse, B, H, bias=None, kv_len=None, causal=False, drop_p=0.0, keep_bits=None):
+    """Fused attention forward (head dim 64, bf16/fp16).  q, ctx: [B*Tq, H*64] views; k, v: [B*Tk, H*64] views; lse fp32
+    [B, H, Tq]; bias fp32 [B, Tk]; kv_len int32 [B]; keep_bits uint8 [B*H*Tq*round8(Tk) / 8] (bit j of byte g = element
+    8g+j).  Writes ctx and lse."""
+    nq, q_ld = _rows(q, H * 64)
+    nk, k_ld = _rows(k, H * 64)
+    _, v_ld = _rows(v, H * 64)
+    _, ctx_ld = _rows(ctx, H * 64)
+    check(load().b200st_attention_fwd(_dt(q), q.data_ptr(), q_ld, k.data_ptr(), k_ld, v.data_ptr(), v_ld, B, H, nq // B, nk // B,
+                                      _ptr(bias), _ptr(kv_len), int(causal), drop_p, _ptr(keep_bits), ctx.data_ptr(), ctx_ld,
+                                      lse.data_ptr(), _stream()))
+    return ctx, lse
+
+
+def attention_bwd(q, k, v, ctx, dctx, lse, dq, dk, dv, dq_scratch, B, H, bias=None, kv_len=None, causal=False, drop_p=0.0,
+                  keep_bits=None):
+    """Fused attention backward: dq [B*Tq, H*64], dk / dv [B*Tk, H*64] views written from ctx / lse of the forward pass
+    and dctx; dq_scratch fp32 with B*Tq*H*64 + B*H*Tq elements."""
+    nq, q_ld = _rows(q, H * 64)
+    nk, k_ld = _rows(k, H * 64)
+    _, v_ld = _rows(v, H * 64)
+    _, ctx_ld = _rows(ctx, H * 64)
+    _, dctx_ld = _rows(dctx, H * 64)
+    _, dq_ld = _rows(dq, H * 64)
+    _, dk_ld = _rows(dk, H * 64)
+    _, dv_ld = _rows(dv, H * 64)
+    Tq = nq // B
+    assert dq_scratch.dtype.itemsize == 4 and dq_scratch.numel() >= B * Tq * H * 64 + B * H * Tq
+    check(load().b200st_attention_bwd(_dt(q), q.data_ptr(), q_ld, k.data_ptr(), k_ld, v.data_ptr(), v_ld, B, H, Tq, nk // B,
+                                      _ptr(bias), _ptr(kv_len), int(causal), drop_p, _ptr(keep_bits), ctx.data_ptr(), ctx_ld,
+                                      dctx.data_ptr(), dctx_ld, lse.data_ptr(), dq_scratch.data_ptr(), dq.data_ptr(), dq_ld,
+                                      dk.data_ptr(), dk_ld, dv.data_ptr(), dv_ld, _stream()))
+    return dq, dk, dv
+
+
+def ffn_fwd(X, W1, b1, W2, b2, F1, x_out, drop_ffn_p=0.0, ffn_bits=None, drop_post_p=0.0, post_bits=None, tickets=None):
+    """Fused FFN forward on packed row-major tensors: F1 [M, ffn] = dropout(relu(X W1 + b1)); x_out fp32 [M, d] +=
+    post-dropout(F1 W2 + b2).  X [M, d], W1 [d, ffn], W2 [ffn, d] bf16/fp16.  Returns the number of hidden slices."""
+    M, d = X.shape
+    ffn = W1.shape[1]
+    for t in (X, W1, W2, F1, x_out):
+        assert t.is_contiguous()
+    splits = C.c_int32(0)
+    check(load().b200st_ffn_fwd(_dt(X), X.data_ptr(), M, d, ffn, W1.data_ptr(), _ptr(b1), W2.data_ptr(), _ptr(b2), drop_ffn_p,
+                                _ptr(ffn_bits), drop_post_p, _ptr(post_bits), F1.data_ptr(), x_out.data_ptr(), _ptr(tickets),
+                                C.byref(splits), _stream()))
+    return splits.value
+
+
+def ffn_bwd(dY, W1, W2, F1, scale, dF1, dH, tickets=None):
+    """Fused FFN data gradient: dF1 [M, ffn] = scale * (dY W2^T) where F1 > 0; dH fp32 [M, d] += dF1 W1^T.
+    Returns the number of hidden slices."""
+    M, d = dY.shape
+    ffn = W1.shape[1]
+    for t in (dY, W1, W2, F1, dF1, dH):
+        assert t.is_contiguous()
+    splits = C.c_int32(0)
+    check(load().b200st_ffn_bwd(_dt(dY), dY.data_ptr(), M, d, ffn, W1.data_ptr(), W2.data_ptr(), F1.data_ptr(), scale,
+                                dF1.data_ptr(), dH.data_ptr(), _ptr(tickets), C.byref(splits), _stream()))
+    return splits.value
 
 
 def profile_begin():
